@@ -21,6 +21,9 @@ over one batch of synthetic frame pairs.  Workload at every N: 512 independent 6
            is absent) = the oracle's scalar FAITHFUL restatement.
   --impl reference: the same CPU implementation from host images (pyramid build + match), all host threads.
   --config 5: BASELINE.json configs[4] (1280x960, 6 levels, mu = 0.05, 32 pairs per GPU = 256 over 8 GPUs).
+  --dump-outputs DIR: after the timed steps, the result records of the last timed step (every pair of the global batch,
+           in pair order) as DIR/<field>.npy in float64, so that two builds can be compared output for output: the inputs
+           are seeded and the same for the same arguments.
 """
 from __future__ import annotations
 
@@ -36,6 +39,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree it runs from
 
 import numpy as np  # noqa: E402
 
@@ -92,7 +96,25 @@ def parse_args():
     ap.add_argument("--cpu-sample", type=int, default=0, help="pairs in the CPU baseline sample (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-consecutive", action="store_true", help="skip the consecutive-frames e2e leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<field>.npy (float64)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+def dump_outputs(directory: str, records: np.ndarray, num_levels: int):
+    """records: dvo_b200_result records (numpy view with the dtype of engine.CResult), one per pair.  Writes every field a
+    caller of dvo_b200_match_batch receives, as float64, the per-level statistics for the levels the configuration runs."""
+    os.makedirs(directory, exist_ok=True)
+    out = {name: records[name] for name in records.dtype.names if name != "levels"}
+    out["transformation"] = out["transformation"].reshape(-1, 4, 4)
+    out["information"] = out["information"].reshape(-1, 6, 6)
+    levels = records["levels"][:, :num_levels]
+    for name in levels.dtype.names:
+        out["levels_" + name] = levels[name]
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -414,6 +436,9 @@ def run_ours(args, rank, local_rank, world):
         res = tensor_to_results(last["gathered"][rank * B:(rank + 1) * B])
     else:
         res = last["res"]
+    if args.dump_outputs and rank == 0:
+        records = last["gathered"].numpy().view(np.dtype(CResult)).reshape(-1) if world > 1 else np.frombuffer(res, dtype=np.dtype(CResult))
+        dump_outputs(args.dump_outputs, records, FIRST_LEVEL - LAST_LEVEL + 1)
     pix_iters = 0
     it_hist = [0] * LEVELS
     for i in range(B):

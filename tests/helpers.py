@@ -1,3 +1,4 @@
+import hashlib
 import os
 
 import numpy as np
@@ -5,6 +6,8 @@ import numpy as np
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 GOLDEN_SEEDS = (11, 12, 13)
 GOLDEN_LEVELS = 3
+# outputs of the original dvo_core's own SSE object code on the golden pairs (tests/golden/make_reference_golden.py)
+REFERENCE_GOLDEN = os.path.join(GOLDEN_DIR, "reference_pin.npz")
 
 # Stated SE(3) tolerance of the path (DESIGN.md "Parity").  Measured with scripts/oracle_spread.py over 96
 # seeded 640x480 pairs: the reference's own numerical noise (_mm_rcp_ps, round-toward-zero, fp32 serial
@@ -39,3 +42,11 @@ def pose_delta(Ta, Tb):
 
 def nan_equal(a, b):
     return np.array_equal(np.isnan(a), np.isnan(b)) and np.array_equal(a[~np.isnan(a)], b[~np.isnan(b)])
+
+
+def nan_digest(a):
+    """sha256 of a float32 array with every NaN made the same NaN and -0 made +0: two arrays have the same digest
+    exactly when nan_equal(a, b) holds and their shapes agree."""
+    a = np.asarray(a, dtype=np.float32)
+    c = np.where(np.isnan(a), np.float32(np.nan), a + np.float32(0.0)).astype(np.float32)
+    return hashlib.sha256(str(c.shape).encode() + np.ascontiguousarray(c).tobytes()).hexdigest()
