@@ -54,13 +54,57 @@ static void drain_profile(dvo_b200_ctx* ctx) {
 
 namespace {
 
-__global__ void k_convert_bgr(const uint8_t* __restrict__ bgr, uint8_t* __restrict__ grey, int n) {
+__global__ void k_convert_bgr(const uint8_t* __restrict__ bgr, size_t row_bytes, size_t image_bytes, uint8_t* __restrict__ grey,
+                              int w, int h) {
   // benchmark_slam.cpp:58-68: cv::cvtColor(rgb, grey, CV_BGR2GRAY) on CV_8UC3 (convertTo(CV_32F) happens in the pyramid
-  // kernels' loads).  OpenCV's 8-bit path is fixed point: (B*1868 + G*9617 + R*4899 + (1 << 13)) >> 14.
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const uint8_t* p = bgr + 3 * (size_t)i;
-  grey[i] = (uint8_t)((1868 * (int)p[0] + 9617 * (int)p[1] + 4899 * (int)p[2] + 8192) >> 14);
+  // kernels' loads).  OpenCV's 8-bit path is fixed point: (B*1868 + G*9617 + R*4899 + (1 << 13)) >> 14.  The BGR frames
+  // are read at their byte strides; the grey images are written dense.
+  const int img = blockIdx.y;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= w * h) return;
+  const int y = i / w, x = i - y * w;
+  const uint8_t* p = bgr + img * image_bytes + (size_t)y * row_bytes + 3 * (size_t)x;
+  grey[(size_t)img * w * h + i] = (uint8_t)((1868 * (int)p[0] + 9617 * (int)p[1] + 4899 * (int)p[2] + 8192) >> 14);
+}
+
+void convert_bgr(dvo_b200_ctx* ctx, const uint8_t* bgr, size_t row_bytes, size_t image_bytes, uint8_t* grey, int n, int w, int h) {
+  k_convert_bgr<<<dim3((unsigned)(((size_t)w * h + 255) / 256), n), 256, 0, ctx->stream>>>(bgr, row_bytes, image_bytes, grey, w, h);
+  ctx->launches++;
+}
+
+// device frames: device or managed memory of the context's device (no host memory, no silent copy)
+int check_device_pointer(dvo_b200_ctx* ctx, const void* p, const std::string& what) {
+  cudaPointerAttributes a;
+  const cudaError_t e = cudaPointerGetAttributes(&a, p);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, what + ": not a CUDA pointer (" + cudaGetErrorString(e) + ")");
+  }
+  if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, what + ": host memory; device or managed memory of the context's device required");
+  if (a.device != ctx->device)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, what + ": memory of device " + std::to_string(a.device) +
+                                                             ", the context runs on device " + std::to_string(ctx->device));
+  return 0;
+}
+
+// one plane of dvo_b200_device_frames: minimum strides and element alignment
+int check_plane(dvo_b200_ctx* ctx, const char* name, const void* p, int64_t row_bytes, int64_t image_bytes, int n, int width,
+                int height, int pixel_bytes, int elem_bytes) {
+  const std::string f = std::string("pyramid_create_device_batch: frames->") + name;
+  if (!p) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + " is null");
+  if (row_bytes < (int64_t)width * pixel_bytes)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + "_row_bytes " + std::to_string(row_bytes) + " < width x " +
+                                                             std::to_string(pixel_bytes) + " bytes");
+  if (n > 1 && image_bytes < (int64_t)height * row_bytes)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + "_image_bytes " + std::to_string(image_bytes) + " < height x " + name +
+                                                             "_row_bytes");
+  if ((uintptr_t)p % elem_bytes) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + " is not " + std::to_string(elem_bytes) + "-byte aligned");
+  if (row_bytes % elem_bytes)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + "_row_bytes is not a multiple of " + std::to_string(elem_bytes));
+  if (n > 1 && image_bytes % elem_bytes)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + "_image_bytes is not a multiple of " + std::to_string(elem_bytes));
+  return check_device_pointer(ctx, p, f);
 }
 
 }  // namespace
@@ -111,6 +155,7 @@ int dvo_b200_destroy(dvo_b200_ctx* ctx) {
   cudaFree(ws.d_iter_log); cudaFree(ws.d_squads);
   if (ws.h_active) cudaFreeHost(ws.h_active);
   pool_close(ctx);
+  tracker_release(ctx);
   cudaFree(ctx->d_stage);
   if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
   if (ctx->h_results) cudaFreeHost(ctx->h_results);
@@ -180,7 +225,8 @@ int dvo_b200_pyramid_create_raw_batch(dvo_b200_ctx* ctx, int32_t n, const uint8_
   DVO_CUDA(ctx, cudaMemcpyAsync(dR, raw_depth, npx * 2, cudaMemcpyHostToDevice, ctx->stream));
   DVO_CUDA(ctx, cudaMemcpyAsync(dG, grey, npx, cudaMemcpyHostToDevice, ctx->stream));
   ctx->h2d_bytes += npx * 3;
-  return pyramid_build_batch_input(ctx, n, dG, dR, 1, depth_scale, width, height, fx, fy, ox, oy, levels, 0.f, 0.f, out);
+  return pyramid_build_batch_input(ctx, n, dense_frames(dG, dR, 1, depth_scale, width, height), width, height, fx, fy, ox, oy, levels,
+                                   0.f, 0.f, out);
 }
 
 int dvo_b200_pyramid_create_bgr_batch(dvo_b200_ctx* ctx, int32_t n, const uint8_t* bgr, const uint16_t* raw_depth,
@@ -199,15 +245,46 @@ int dvo_b200_pyramid_create_bgr_batch(dvo_b200_ctx* ctx, int32_t n, const uint8_
   DVO_CUDA(ctx, cudaMemcpyAsync(dR, raw_depth, npx * 2, cudaMemcpyHostToDevice, ctx->stream));
   DVO_CUDA(ctx, cudaMemcpyAsync(dC, bgr, npx * 3, cudaMemcpyHostToDevice, ctx->stream));
   ctx->h2d_bytes += npx * 5;
-  k_convert_bgr<<<(unsigned)((npx + 255) / 256), 256, 0, ctx->stream>>>(dC, dG, (int)npx);   // 8-bit grey, as cv::cvtColor leaves it
-  ctx->launches++;
-  return pyramid_build_batch_input(ctx, n, dG, dR, 1, depth_scale, width, height, fx, fy, ox, oy, levels, 0.f, 0.f, out);
+  convert_bgr(ctx, dC, (size_t)width * 3, (size_t)width * height * 3, dG, n, width, height);   // 8-bit grey, as cv::cvtColor leaves it
+  return pyramid_build_batch_input(ctx, n, dense_frames(dG, dR, 1, depth_scale, width, height), width, height, fx, fy, ox, oy, levels,
+                                   0.f, 0.f, out);
 }
 
 int dvo_b200_pyramid_create_raw(dvo_b200_ctx* ctx, const uint8_t* grey, const uint16_t* raw_depth, float depth_scale,
                                 int32_t width, int32_t height, float fx, float fy, float ox, float oy, int32_t levels,
                                 dvo_b200_pyramid** out) {
   return dvo_b200_pyramid_create_raw_batch(ctx, 1, grey, raw_depth, depth_scale, width, height, fx, fy, ox, oy, levels, out);
+}
+
+int dvo_b200_pyramid_create_device_batch(dvo_b200_ctx* ctx, int32_t n, const dvo_b200_device_frames* frames, float fx, float fy,
+                                         float ox, float oy, int32_t levels, dvo_b200_pyramid** out) {
+  if (!ctx || !frames || !out || n <= 0)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "pyramid_create_device_batch: null/invalid argument");
+  const dvo_b200_device_frames& f = *frames;
+  if (f.format < DVO_B200_FRAME_F32 || f.format > DVO_B200_FRAME_BGR8_RAW16)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "pyramid_create_device_batch: frames->format " + std::to_string(f.format) + " is unknown");
+  if (f.width <= 0 || f.height <= 0)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "pyramid_create_device_batch: frames->width / height must be positive");
+  cudaSetDevice(ctx->device);
+  const bool f32 = f.format == DVO_B200_FRAME_F32;
+  const int colour_px = f32 ? 4 : (f.format == DVO_B200_FRAME_GREY8_RAW16 ? 1 : 3), colour_elem = f32 ? 4 : 1;
+  const int depth_px = f32 ? 4 : 2;
+  int rc = check_plane(ctx, "colour", f.colour, f.colour_row_bytes, f.colour_image_bytes, n, f.width, f.height, colour_px, colour_elem);
+  if (!rc) rc = check_plane(ctx, "depth", f.depth, f.depth_row_bytes, f.depth_image_bytes, n, f.width, f.height, depth_px, depth_px);
+  if (rc) return rc;
+  FrameInput in;
+  in.I = f.colour; in.i_row = (size_t)f.colour_row_bytes; in.i_img = n > 1 ? (size_t)f.colour_image_bytes : 0;
+  in.Z = f.depth; in.z_row = (size_t)f.depth_row_bytes; in.z_img = n > 1 ? (size_t)f.depth_image_bytes : 0;
+  in.raw = f32 ? 0 : 1; in.zscale = f32 ? 0.f : f.depth_scale;
+  if (f.format == DVO_B200_FRAME_BGR8_RAW16) {
+    // grey into the staging area, as the host path leaves it; then the raw path reads it dense
+    const size_t npx = (size_t)f.width * f.height * n;
+    if ((rc = ensure_stage(ctx, npx + 64, 0))) return rc;
+    uint8_t* dG = (uint8_t*)ctx->d_stage;
+    convert_bgr(ctx, (const uint8_t*)f.colour, in.i_row, in.i_img, dG, n, f.width, f.height);
+    in.I = dG; in.i_row = (size_t)f.width; in.i_img = (size_t)f.width * f.height;
+  }
+  return pyramid_build_batch_input(ctx, n, in, f.width, f.height, fx, fy, ox, oy, levels, 0.f, 0.f, out);
 }
 
 int dvo_b200_pyramid_device(const dvo_b200_pyramid* p) { return p ? p->device : -1; }
@@ -313,6 +390,20 @@ int dvo_b200_match_batch_device(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, i
   if (!ctx || !d_results) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_device: null argument");
   cudaSetDevice(ctx->device);
   return tracker_match_batch(ctx, cfg, n, references, currents, T_init, nullptr, d_results, nullptr, 0);
+}
+
+int dvo_b200_match_batch_enqueue(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int32_t n, dvo_b200_pyramid* const* references,
+                                 dvo_b200_pyramid* const* currents, const double* d_T_init, void* d_results) {
+  if (!ctx || !d_results) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_enqueue: null argument");
+  cudaSetDevice(ctx->device);
+  if ((uintptr_t)d_results % 8) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_enqueue: d_results is not 8-byte aligned");
+  int rc = check_device_pointer(ctx, d_results, "match_batch_enqueue: d_results");
+  if (rc) return rc;
+  if (cfg && cfg->use_initial_estimate && d_T_init) {
+    if ((uintptr_t)d_T_init % 8) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_enqueue: d_T_init is not 8-byte aligned");
+    if ((rc = check_device_pointer(ctx, d_T_init, "match_batch_enqueue: d_T_init"))) return rc;
+  }
+  return tracker_match_batch(ctx, cfg, n, references, currents, d_T_init, nullptr, d_results, nullptr, 0, true);
 }
 
 int dvo_b200_residual_image(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, dvo_b200_pyramid* reference,

@@ -171,6 +171,7 @@ struct Workspace {              // per-ctx scratch of the level kernel
   double* d_tinit = nullptr;         // per pair initial estimate (4x4)
   dvo_b200_iteration_stats* d_iter_log = nullptr;
   int* h_active = nullptr;           // pinned: per level, the kernel's error flag
+  int* h_flag_accum = nullptr;       // pinned: a timeout code not yet reported (enqueued launches fold their flag in here)
   char* d_squads = nullptr;          // persistent kernel: SquadState[nsquads] + {queue head, error flag}
   size_t cap_pairs = 0, cap_row_exports = 0, cap_row_base = 0, cap_strip_exports = 0, cap_strip_base = 0, cap_row_partial = 0, cap_strip_partial = 0,
          cap_squads = 0, cap_iter_log = 0, cap_dump = 0, cap_tinit = 0;
@@ -187,6 +188,14 @@ struct dvo_b200_ctx {
   std::string last_error;
   int64_t launches = 0, h2d_bytes = 0, d2h_bytes = 0;
   int pending_level_flags = 0;          // levels whose error flag has been copied to pinned memory but not yet checked
+  // pinned pair-descriptor slots of dvo_b200_match_batch_enqueue, used round robin: a slot is rewritten only once the event
+  // recorded after the k_stage_words that read it has completed, so the host waits only when the ring wraps onto a slot
+  // still in flight
+  static constexpr int kDescSlots = 4;
+  void* h_desc[kDescSlots] = {};
+  cudaEvent_t desc_staged[kDescSlots] = {};
+  size_t desc_slot_bytes = 0;
+  int desc_next = 0;
   uint64_t next_pyramid_id = 1;
   dvo_b200::Workspace ws;
   std::shared_ptr<dvo_b200::SlabPool> pool;   // pooled device slabs (see SlabPool)
@@ -221,21 +230,39 @@ struct ProfScope {
   ~ProfScope();
 };
 
+// Level-0 input frames of a pyramid build, in device memory, addressed in bytes: pixel (x, y) of image i of the intensity
+// lies at I + i * i_img + y * i_row + x * (pixel size), likewise for the depth.  raw == 0: float32 intensity / float32 depth
+// in metres (NaN = invalid); raw == 1: 8-bit grey / 16-bit raw depth (depth = raw * zscale, 0 -> NaN).  The host entry
+// points stage dense images (dense_frames); device-input callers pass their own pitches.
+struct FrameInput {
+  const void* I = nullptr;
+  const void* Z = nullptr;
+  size_t i_row = 0, i_img = 0, z_row = 0, z_img = 0;
+  int raw = 0;
+  float zscale = 0.f;
+};
+
 // pyramid.cu
+FrameInput dense_frames(const void* d_I, const void* d_Z, int raw, float zscale, int w, int h);
 int pyramid_build_batch(dvo_b200_ctx* ctx, int n, const float* d_I, const float* d_Z, int w, int h, float fx, float fy,
                         float ox, float oy, int levels, float ti, float td, dvo_b200_pyramid** out);
-int pyramid_build_batch_input(dvo_b200_ctx* ctx, int n, const void* d_I, const void* d_Z, int raw, float zscale, int w, int h,
-                              float fx, float fy, float ox, float oy, int levels, float ti, float td, dvo_b200_pyramid** out);
+int pyramid_build_batch_input(dvo_b200_ctx* ctx, int n, const FrameInput& in, int w, int h, float fx, float fy, float ox, float oy,
+                              int levels, float ti, float td, dvo_b200_pyramid** out);
 int pyramid_reselect(dvo_b200_ctx* ctx, dvo_b200_pyramid* p, float ti, float td);
 void pyramid_free(dvo_b200_pyramid* p);
 void pool_close(dvo_b200_ctx* ctx);
 int ensure_stage(dvo_b200_ctx* ctx, size_t dev_bytes, size_t host_bytes);
 
 // tracker.cu
+// enqueue = false: T_init is host memory (staged with the descriptors); the call waits for the previous use of the pinned
+// stage and, with h_results, for the results.  enqueue = true (dvo_b200_match_batch_enqueue): T_init and d_results are
+// device memory, the descriptors go through the slot ring and the host does not wait for the GPU.
 int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dvo_b200_pyramid* const* refs,
                         dvo_b200_pyramid* const* curs, const double* T_init, dvo_b200_result* h_results,
-                        void* d_results, dvo_b200_iteration_stats* iter_stats, int max_iter_stats);
+                        void* d_results, dvo_b200_iteration_stats* iter_stats, int max_iter_stats, bool enqueue = false);
 int check_level_flags(dvo_b200_ctx* ctx);   // after a stream synchronisation: did a level kernel report a timeout?
+void fold_level_flags(dvo_b200_ctx* ctx);   // after a stream synchronisation: keep reported timeouts for check_level_flags
+void tracker_release(dvo_b200_ctx* ctx);    // frees the tracker's pinned buffers and events (stream synchronised)
 int tracker_linearize(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, dvo_b200_pyramid* ref, dvo_b200_pyramid* cur,
                       int level, const double* T, int use_weights, const float* prev_precision, int64_t* count,
                       float* precision_out, float* ll_out, double* A_out, double* b_out, float* planes7);

@@ -18,27 +18,30 @@ __device__ __forceinline__ bool is_nan(float v) { return v != v; }
 // benchmark_slam.cpp:46-93 hands to RgbdCameraPyramid::create.  kRaw = true: 8-bit grey and 16-bit raw depth straight from
 // the image files; the loader's conversions -- convertTo(CV_32F) and SurfacePyramid::convertRawDepthImageSse
 // (surface_pyramid.cpp:65-105: u16 * scale, 0 -> NaN) -- happen in the load, no float32 copy of the frame is ever written.
+// The input images are addressed in bytes (FrameInput: row and image strides), so a pitched or sliced frame is read in
+// place; `off` is the byte offset of the pixel from `base`.
 template <bool kRaw>
-__device__ __forceinline__ float load_intensity(const void* I, size_t i) {
-  if (kRaw) return (float)__ldg(reinterpret_cast<const uint8_t*>(I) + i);
-  return __ldg(reinterpret_cast<const float*>(I) + i);
+__device__ __forceinline__ float load_intensity(const char* base, size_t off) {
+  if (kRaw) return (float)__ldg(reinterpret_cast<const uint8_t*>(base + off));
+  return __ldg(reinterpret_cast<const float*>(base + off));
 }
 template <bool kRaw>
-__device__ __forceinline__ float load_depth(const void* Z, size_t i, float scale) {
+__device__ __forceinline__ float load_depth(const char* base, size_t off, float scale) {
   if (kRaw) {
-    const uint16_t r = __ldg(reinterpret_cast<const uint16_t*>(Z) + i);
+    const uint16_t r = __ldg(reinterpret_cast<const uint16_t*>(base + off));
     return r == 0 ? __int_as_float(0x7fc00000) : __fmul_rn((float)r, scale);
   }
-  return __ldg(reinterpret_cast<const float*>(Z) + i);
+  return __ldg(reinterpret_cast<const float*>(base + off));
 }
+template <bool kRaw> constexpr int intensity_bytes() { return kRaw ? 1 : 4; }
+template <bool kRaw> constexpr int depth_bytes() { return kRaw ? 2 : 4; }
 
 // level l intensity = ((a+b)+c)+d)/4 of the 2x2 block of level l-1 (rgbd_image.cpp:38-55), into P0.x (the Z slot is
-// filled by the finish pass).  kFromInput: level 1 reads the input image, which is level 0's intensity.
-// sp / dp: row pitch of the source / destination planes (float2 elements).
+// filled by the finish pass).  kFromInput: level 1 reads the input image, which is level 0's intensity, at byte strides
+// in_row / in_img.  sp / dp: row pitch of the source / destination planes (float2 elements).
 template <bool kFromInput, bool kRaw>
-__global__ void k_pyr_intensity_down(const void* __restrict__ I0, size_t in_stride, int aligned, float2* __restrict__ planes,
-                                     size_t planes_per_image, size_t src_off, int sw, int sp, size_t dst_off, int dw, int dh,
-                                     int dp) {
+__global__ void k_pyr_intensity_down(const void* __restrict__ I0, size_t in_row, size_t in_img, int aligned, float2* __restrict__ planes,
+                                     size_t planes_per_image, size_t src_off, int sp, size_t dst_off, int dw, int dh, int dp) {
   int img = blockIdx.y;
   int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= dw * dh) return;
@@ -46,22 +49,21 @@ __global__ void k_pyr_intensity_down(const void* __restrict__ I0, size_t in_stri
   float2* D = planes + img * planes_per_image + dst_off;
   float a, b, c, d;
   if (kFromInput) {
-    const size_t i0 = (size_t)img * in_stride + (size_t)(2 * y) * sw + 2 * x;
+    const char* r0 = reinterpret_cast<const char*>(I0) + img * in_img + (size_t)(2 * y) * in_row + (size_t)(2 * x) * intensity_bytes<kRaw>();
+    const char* r1 = r0 + in_row;
     if (kRaw) {
-      const uint8_t* g = reinterpret_cast<const uint8_t*>(I0) + i0;
-      if (aligned) {   // even width and image stride: every 2x2 block starts 2-byte aligned
-        const uchar2 u = __ldg(reinterpret_cast<const uchar2*>(g)), v = __ldg(reinterpret_cast<const uchar2*>(g + sw));
+      if (aligned) {   // base, row and image strides even: every 2x2 block starts 2-byte aligned
+        const uchar2 u = __ldg(reinterpret_cast<const uchar2*>(r0)), v = __ldg(reinterpret_cast<const uchar2*>(r1));
         a = (float)u.x; b = (float)u.y; c = (float)v.x; d = (float)v.y;
       } else {
-        a = (float)__ldg(g); b = (float)__ldg(g + 1); c = (float)__ldg(g + sw); d = (float)__ldg(g + sw + 1);
+        a = load_intensity<true>(r0, 0); b = load_intensity<true>(r0, 1); c = load_intensity<true>(r1, 0); d = load_intensity<true>(r1, 1);
       }
     } else {
-      const float* p0 = reinterpret_cast<const float*>(I0) + i0;
-      if (aligned) {   // even width and image stride: every 2x2 block starts 8-byte aligned
-        const float2 u = __ldg(reinterpret_cast<const float2*>(p0)), v = __ldg(reinterpret_cast<const float2*>(p0 + sw));
+      if (aligned) {   // base, row and image strides multiples of 8 bytes: every 2x2 block starts 8-byte aligned
+        const float2 u = __ldg(reinterpret_cast<const float2*>(r0)), v = __ldg(reinterpret_cast<const float2*>(r1));
         a = u.x; b = u.y; c = v.x; d = v.y;
       } else {
-        a = __ldg(p0); b = __ldg(p0 + 1); c = __ldg(p0 + sw); d = __ldg(p0 + sw + 1);
+        a = load_intensity<false>(r0, 0); b = load_intensity<false>(r0, 4); c = load_intensity<false>(r1, 0); d = load_intensity<false>(r1, 4);
       }
     }
   } else {
@@ -79,13 +81,13 @@ __global__ void k_pyr_intensity_down(const void* __restrict__ I0, size_t in_stri
 // gradients (clamped central differences), masked and true depth, default selection mask and reference plane
 // (I, Zsel: depth where the pixel is selected, NaN elsewhere) for one level.
 // Depth of level l is the pure subsample chain of level 0 (rgbd_image.cpp:127-139): Z_l(y,x) = Z_0(y<<l, x<<l).
-// Level 0 reads its intensity straight from the input image I0 (no intermediate copy); the other levels read the
-// intensity that k_pyr_intensity_down left in P0.x.  The selection count / last selected index are derived from
-// the masks afterwards (k_sel_info): no atomics here.  Threads walk the linear pixel index y*w+x (the order of the
+// Level 0 reads its intensity straight from the input image (no intermediate copy); the other levels read the
+// intensity that k_pyr_intensity_down left in P0.x.  Input taps are addressed with the byte strides of `src`.  The
+// selection count / last selected index are derived from the masks afterwards (k_sel_info): no atomics here.  Threads walk the linear pixel index y*w+x (the order of the
 // selection mask); the planes are addressed with the row pitch.
 template <bool kLevel0, bool kRaw>
 __global__ void __launch_bounds__(256)
-k_pyr_finish(const void* __restrict__ I0, const void* __restrict__ Z0, float zscale, int w0, int n0, float2* __restrict__ planes,
+k_pyr_finish(const FrameInput src, float2* __restrict__ planes,
              size_t planes_per_image, size_t plane_off, size_t rec_off, int nbands, int w, int h, int pitch, int level,
              uint32_t* __restrict__ masks, size_t mask_words_per_image, size_t mask_off, float ti, float td) {
   const int img = blockIdx.y;
@@ -99,12 +101,15 @@ k_pyr_finish(const void* __restrict__ I0, const void* __restrict__ Z0, float zsc
     float2* P0 = planes + img * planes_per_image + plane_off;
     float2* P2 = P0 + plane;   // P2 = (I, Z); the depth gradients are not stored
     float2* rec = planes + img * planes_per_image + rec_off;   // reference tile records: (I, Zsel) and (Ix, Iy)
-    const size_t zb = (size_t)img * n0;
+    const char* Ib = reinterpret_cast<const char*>(src.I) + img * src.i_img;
+    const char* Zb = reinterpret_cast<const char*>(src.Z) + img * src.z_img;
     const int xp = max(x - 1, 0), xn = min(x + 1, w - 1), yp = max(y - 1, 0), yn = min(y + 1, h - 1);
     float I, ixp, ixn, iyp, iyn;
     if (kLevel0) {
-      I = load_intensity<kRaw>(I0, zb + idx); ixp = load_intensity<kRaw>(I0, zb + y * w + xp); ixn = load_intensity<kRaw>(I0, zb + y * w + xn);
-      iyp = load_intensity<kRaw>(I0, zb + yp * w + x); iyn = load_intensity<kRaw>(I0, zb + yn * w + x);
+      constexpr int E = intensity_bytes<kRaw>();
+      const char* row = Ib + (size_t)y * src.i_row;
+      I = load_intensity<kRaw>(row, (size_t)x * E); ixp = load_intensity<kRaw>(row, (size_t)xp * E); ixn = load_intensity<kRaw>(row, (size_t)xn * E);
+      iyp = load_intensity<kRaw>(Ib + (size_t)yp * src.i_row, (size_t)x * E); iyn = load_intensity<kRaw>(Ib + (size_t)yn * src.i_row, (size_t)x * E);
     } else {
       const size_t row = (size_t)y * pitch;
       I = P0[row + x].x; ixp = P0[row + xp].x; ixn = P0[row + xn].x;
@@ -112,11 +117,14 @@ k_pyr_finish(const void* __restrict__ I0, const void* __restrict__ Z0, float zsc
     }
     const float ix = (ixn - ixp) * 0.5f;
     const float iy = (iyn - iyp) * 0.5f;
-    const size_t zr = (size_t)(y << level) * w0;
-    const float z = load_depth<kRaw>(Z0, zb + zr + (x << level), zscale);
-    const float zx = (load_depth<kRaw>(Z0, zb + zr + (xn << level), zscale) - load_depth<kRaw>(Z0, zb + zr + (xp << level), zscale)) * 0.5f;
-    const float zy = (load_depth<kRaw>(Z0, zb + (size_t)(yn << level) * w0 + (x << level), zscale) -
-                      load_depth<kRaw>(Z0, zb + (size_t)(yp << level) * w0 + (x << level), zscale)) * 0.5f;
+    constexpr int EZ = depth_bytes<kRaw>();
+    const float zscale = src.zscale;
+    const char* zr = Zb + (size_t)(y << level) * src.z_row;
+    const size_t zc = (size_t)(x << level) * EZ;
+    const float z = load_depth<kRaw>(zr, zc, zscale);
+    const float zx = (load_depth<kRaw>(zr, (size_t)(xn << level) * EZ, zscale) - load_depth<kRaw>(zr, (size_t)(xp << level) * EZ, zscale)) * 0.5f;
+    const float zy = (load_depth<kRaw>(Zb + (size_t)(yn << level) * src.z_row, zc, zscale) -
+                      load_depth<kRaw>(Zb + (size_t)(yp << level) * src.z_row, zc, zscale)) * 0.5f;
     const bool bad = is_nan(I) || is_nan(ix) || is_nan(iy) || is_nan(z) || is_nan(zx) || is_nan(zy);
     const float zm = bad ? __int_as_float(0x7fc00000) : z;
     const size_t o = (size_t)y * pitch + x;
@@ -319,14 +327,21 @@ void pool_close(dvo_b200_ctx* ctx) {
   ctx->pool->closed = true;
 }
 
-int pyramid_build_batch(dvo_b200_ctx* ctx, int n, const float* d_I, const float* d_Z, int w, int h, float fx, float fy,
-                        float ox, float oy, int levels, float ti, float td, dvo_b200_pyramid** out) {
-  return pyramid_build_batch_input(ctx, n, d_I, d_Z, 0, 0.f, w, h, fx, fy, ox, oy, levels, ti, td, out);
+FrameInput dense_frames(const void* d_I, const void* d_Z, int raw, float zscale, int w, int h) {
+  FrameInput f;
+  f.I = d_I; f.Z = d_Z; f.raw = raw; f.zscale = zscale;
+  f.i_row = (size_t)w * (raw ? 1 : 4); f.i_img = f.i_row * h;
+  f.z_row = (size_t)w * (raw ? 2 : 4); f.z_img = f.z_row * h;
+  return f;
 }
 
-// d_I / d_Z: raw == 0: float32 intensity / float32 depth; raw == 1: 8-bit grey / 16-bit raw depth (depth = raw * zscale, 0 -> NaN)
-int pyramid_build_batch_input(dvo_b200_ctx* ctx, int n, const void* d_I, const void* d_Z, int raw, float zscale, int w, int h,
-                              float fx, float fy, float ox, float oy, int levels, float ti, float td, dvo_b200_pyramid** out) {
+int pyramid_build_batch(dvo_b200_ctx* ctx, int n, const float* d_I, const float* d_Z, int w, int h, float fx, float fy,
+                        float ox, float oy, int levels, float ti, float td, dvo_b200_pyramid** out) {
+  return pyramid_build_batch_input(ctx, n, dense_frames(d_I, d_Z, 0, 0.f, w, h), w, h, fx, fy, ox, oy, levels, ti, td, out);
+}
+
+int pyramid_build_batch_input(dvo_b200_ctx* ctx, int n, const FrameInput& in, int w, int h, float fx, float fy, float ox, float oy,
+                              int levels, float ti, float td, dvo_b200_pyramid** out) {
   if (n <= 0 || levels < 1 || levels > kMaxLevels || w < 32 || h < 2)
     return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "pyramid: bad geometry");
   LevelInfo L[kMaxLevels];
@@ -384,19 +399,22 @@ int pyramid_build_batch_input(dvo_b200_ctx* ctx, int n, const void* d_I, const v
       ctx->launches += 1;
       if (l == 0) continue;   // level 0 takes its intensity from the input image
       dim3 g((q.n + T - 1) / T, n);
-      const int aligned = (((size_t)w * h) | (size_t)w) % 2 == 0 ? 1 : 0;
-      if (l == 1 && raw) k_pyr_intensity_down<true, true><<<g, T, 0, st>>>(d_I, (size_t)w * h, aligned, planes, plane_f2, 0, L[0].w, L[0].pitch, q.plane_off, q.w, q.h, q.pitch);
-      else if (l == 1) k_pyr_intensity_down<true, false><<<g, T, 0, st>>>(d_I, (size_t)w * h, aligned, planes, plane_f2, 0, L[0].w, L[0].pitch, q.plane_off, q.w, q.h, q.pitch);
-      else k_pyr_intensity_down<false, false><<<g, T, 0, st>>>(nullptr, 0, 0, planes, plane_f2, L[l - 1].plane_off, L[l - 1].w, L[l - 1].pitch, q.plane_off, q.w, q.h, q.pitch);
+      // the vector 2x2 loads need every block to start on a multiple of two pixels: base, row stride and (for a batch) image
+      // stride all even multiples of the pixel size
+      const size_t pair_bytes = in.raw ? 2 : 8;
+      const int aligned = (((uintptr_t)in.I | in.i_row | (n > 1 ? in.i_img : 0)) % pair_bytes) == 0 ? 1 : 0;
+      if (l == 1 && in.raw) k_pyr_intensity_down<true, true><<<g, T, 0, st>>>(in.I, in.i_row, in.i_img, aligned, planes, plane_f2, 0, L[0].pitch, q.plane_off, q.w, q.h, q.pitch);
+      else if (l == 1) k_pyr_intensity_down<true, false><<<g, T, 0, st>>>(in.I, in.i_row, in.i_img, aligned, planes, plane_f2, 0, L[0].pitch, q.plane_off, q.w, q.h, q.pitch);
+      else k_pyr_intensity_down<false, false><<<g, T, 0, st>>>(nullptr, 0, 0, 0, planes, plane_f2, L[l - 1].plane_off, L[l - 1].pitch, q.plane_off, q.w, q.h, q.pitch);
       ctx->launches += 1;
     }
     for (int l = 0; l < levels; ++l) {
       const LevelInfo& q = L[l];
       dim3 g((q.words * 32 + T - 1) / T, n);
-      if (l == 0 && raw) k_pyr_finish<true, true><<<g, T, 0, st>>>(d_I, d_Z, zscale, w, w * h, planes, plane_f2, q.plane_off, q.rec_off, q.nbands, q.w, q.h, q.pitch, l, masks, mask_words, q.mask_off, ti, td);
-      else if (l == 0) k_pyr_finish<true, false><<<g, T, 0, st>>>(d_I, d_Z, zscale, w, w * h, planes, plane_f2, q.plane_off, q.rec_off, q.nbands, q.w, q.h, q.pitch, l, masks, mask_words, q.mask_off, ti, td);
-      else if (raw) k_pyr_finish<false, true><<<g, T, 0, st>>>(d_I, d_Z, zscale, w, w * h, planes, plane_f2, q.plane_off, q.rec_off, q.nbands, q.w, q.h, q.pitch, l, masks, mask_words, q.mask_off, ti, td);
-      else k_pyr_finish<false, false><<<g, T, 0, st>>>(d_I, d_Z, zscale, w, w * h, planes, plane_f2, q.plane_off, q.rec_off, q.nbands, q.w, q.h, q.pitch, l, masks, mask_words, q.mask_off, ti, td);
+      if (l == 0 && in.raw) k_pyr_finish<true, true><<<g, T, 0, st>>>(in, planes, plane_f2, q.plane_off, q.rec_off, q.nbands, q.w, q.h, q.pitch, l, masks, mask_words, q.mask_off, ti, td);
+      else if (l == 0) k_pyr_finish<true, false><<<g, T, 0, st>>>(in, planes, plane_f2, q.plane_off, q.rec_off, q.nbands, q.w, q.h, q.pitch, l, masks, mask_words, q.mask_off, ti, td);
+      else if (in.raw) k_pyr_finish<false, true><<<g, T, 0, st>>>(in, planes, plane_f2, q.plane_off, q.rec_off, q.nbands, q.w, q.h, q.pitch, l, masks, mask_words, q.mask_off, ti, td);
+      else k_pyr_finish<false, false><<<g, T, 0, st>>>(in, planes, plane_f2, q.plane_off, q.rec_off, q.nbands, q.w, q.h, q.pitch, l, masks, mask_words, q.mask_off, ti, td);
       k_sel_info<<<n, 32, 0, st>>>(masks, mask_words, q.mask_off, q.words, sel, sel_ints, l);
       k_drop_odd_last<<<(n + 127) / 128, 128, 0, st>>>(planes, plane_f2, q.rec_off, q.nbands, q.w, sel, sel_ints, l, n);
       const int ntiles = q.nbands * q.nstrips;

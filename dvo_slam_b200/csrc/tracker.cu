@@ -118,6 +118,13 @@ __global__ void k_stage_words(const uint4* __restrict__ src, uint4* __restrict__
   if (i < n16) dst[i] = src[i];
 }
 
+// The enqueue-only alignment never waits for the level kernels, and the next launch zeroes a launch's error flag: the flag
+// is folded right after each launch into a pinned word that the next synchronisation reads.
+__global__ void k_fold_flag(const int* __restrict__ flag, int* __restrict__ accum) {
+  const int v = *flag;
+  if (v) *accum = v;
+}
+
 // one warp per pair: combine the strip summaries of the level in order -> covariance -> P_k (dense_tracking.cpp:276-295).
 // e: the level's nstrips strip summaries; strip_base: nstrips + 1 exclusive prefixes of their valid counts (output).
 __device__ __noinline__ void pair_mid_warp(PairState& st, int pair, const double* e, int* strip_base, int nstrips, int* active,
@@ -751,6 +758,10 @@ int ensure_workspace(dvo_b200_ctx* ctx, int npairs, const ScratchNeed& need, int
   if ((rc = grow(ctx, ws.d_squads, ws.cap_squads, need.squads * sizeof(SquadState)))) return rc;
   if ((rc = grow(ctx, ws.d_dump, ws.cap_dump, need.dump_floats))) return rc;
   if (!ws.h_active) DVO_CUDA(ctx, cudaMallocHost((void**)&ws.h_active, sizeof(int) * 8));
+  if (!ws.h_flag_accum) {
+    DVO_CUDA(ctx, cudaMallocHost((void**)&ws.h_flag_accum, sizeof(int)));
+    *ws.h_flag_accum = 0;
+  }
   if (max_log_per_pair > 0) {
     size_t n = (size_t)npairs * max_log_per_pair;
     if ((rc = grow(ctx, ws.d_iter_log, ws.cap_iter_log, n))) return rc;
@@ -991,11 +1002,35 @@ int launch_segments(dvo_b200_ctx* ctx, int nseg, const LevelLaunch (*lps)[kMaxLe
   return 0;
 }
 
+// A pinned slot of at least `bytes` for the pair descriptors of one enqueued call.  Waits only if the ring has wrapped onto
+// a slot whose k_stage_words has not run yet; growing the slots (a larger batch than before) waits for all of them.
+int acquire_desc_slot(dvo_b200_ctx* ctx, size_t bytes, int* slot) {
+  if (bytes > ctx->desc_slot_bytes) {
+    for (int i = 0; i < dvo_b200_ctx::kDescSlots; ++i) {
+      if (ctx->desc_staged[i]) DVO_CUDA(ctx, cudaEventSynchronize(ctx->desc_staged[i]));
+      if (ctx->h_desc[i]) cudaFreeHost(ctx->h_desc[i]);
+      ctx->h_desc[i] = nullptr;
+    }
+    ctx->desc_slot_bytes = 0;
+    for (int i = 0; i < dvo_b200_ctx::kDescSlots; ++i) {
+      DVO_CUDA(ctx, cudaMallocHost(&ctx->h_desc[i], bytes));
+      if (!ctx->desc_staged[i]) DVO_CUDA(ctx, cudaEventCreateWithFlags(&ctx->desc_staged[i], cudaEventDisableTiming));
+    }
+    ctx->desc_slot_bytes = bytes;
+  }
+  const int i = ctx->desc_next;
+  ctx->desc_next = (i + 1) % dvo_b200_ctx::kDescSlots;
+  if (cudaEventQuery(ctx->desc_staged[i]) == cudaErrorNotReady) DVO_CUDA(ctx, cudaEventSynchronize(ctx->desc_staged[i]));
+  cudaGetLastError();
+  *slot = i;
+  return 0;
+}
+
 }  // namespace
 
 int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dvo_b200_pyramid* const* refs,
                         dvo_b200_pyramid* const* curs, const double* T_init, dvo_b200_result* h_results,
-                        void* d_results_user, dvo_b200_iteration_stats* iter_stats, int max_iter_stats) {
+                        void* d_results_user, dvo_b200_iteration_stats* iter_stats, int max_iter_stats, bool enqueue) {
   int rc = check_batch(ctx, cfg, n, refs, curs);
   if (rc) return rc;
   cudaStream_t st = ctx->stream;
@@ -1074,29 +1109,52 @@ int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dv
 
   // Pair descriptors of every level and the initial estimates go into the pinned stage once; one small kernel copies
   // them to device memory (reads over PCIe: no H2D copy-engine work, no host round trip between the launches below).
+  // The enqueue variant takes the initial estimates from the caller's device memory and stages only the descriptors, in
+  // a slot of the descriptor ring.
   const size_t desc_bytes = (sizeof(PairLevel) * (size_t)n * nlev + 15) / 16 * 16;
   const bool have_init = cfg->use_initial_estimate && T_init;
-  const size_t init_bytes = have_init ? sizeof(double) * 16 * (size_t)n : 0;
-  if ((rc = ensure_stage(ctx, 0, desc_bytes + init_bytes))) return rc;
-  if ((rc = grow(ctx, ws.d_tinit, ws.cap_tinit, (size_t)16 * n))) return rc;
-  DVO_CUDA(ctx, cudaStreamSynchronize(st));   // previous use of the pinned stage has drained
-  PairLevel* h_desc = (PairLevel*)ctx->h_stage;
+  const size_t init_bytes = have_init && !enqueue ? sizeof(double) * 16 * (size_t)n : 0;
+  PairLevel* h_desc = nullptr;
+  int slot = 0;
+  if (enqueue) {
+    if ((rc = acquire_desc_slot(ctx, desc_bytes, &slot))) return rc;
+    h_desc = (PairLevel*)ctx->h_desc[slot];
+  } else {
+    if ((rc = ensure_stage(ctx, 0, desc_bytes + init_bytes))) return rc;
+    if ((rc = grow(ctx, ws.d_tinit, ws.cap_tinit, (size_t)16 * n))) return rc;
+    DVO_CUDA(ctx, cudaStreamSynchronize(st));   // previous use of the pinned stage has drained
+    fold_level_flags(ctx);                      // flags of an earlier call whose results stayed on the device
+    h_desc = (PairLevel*)ctx->h_stage;
+    if (have_init) std::memcpy((char*)ctx->h_stage + desc_bytes, T_init, init_bytes);
+  }
   for (int level = first, li = 0; level >= last; --level, ++li) fill_pair_levels(h_desc + (size_t)li * n, n, refs, curs, level);
-  if (have_init) std::memcpy((char*)ctx->h_stage + desc_bytes, T_init, init_bytes);
   ctx->h2d_bytes += desc_bytes + init_bytes;
   {
     ProfScope prof(ctx, 2);
     const size_t n16 = desc_bytes / 16;
     k_stage_words<<<(unsigned)((n16 + 255) / 256), 256, 0, st>>>((const uint4*)h_desc, (uint4*)ws.d_pair_level, n16);
     ctx->launches++;
-    if (have_init) {
+    if (init_bytes) {
       const size_t m16 = init_bytes / 16;
       k_stage_words<<<(unsigned)((m16 + 255) / 256), 256, 0, st>>>((const uint4*)((char*)ctx->h_stage + desc_bytes), (uint4*)ws.d_tinit, m16);
       ctx->launches++;
     }
   }
+  if (enqueue) DVO_CUDA(ctx, cudaEventRecord(ctx->desc_staged[slot], st));
+  else for (int i = 0; i < 8; ++i) ws.h_active[i] = 0;
+  const double* d_tinit = !have_init ? nullptr : enqueue ? T_init : ws.d_tinit;
+  // after each launch its error flag goes to pinned memory: into the per-level slots checked when this call (or the next
+  // synchronisation) waits, or -- enqueue -- folded into the word the next synchronisation reads
+  auto keep_flag = [&](int launch, int* flag) -> int {
+    if (enqueue) {
+      k_fold_flag<<<1, 1, 0, st>>>(flag, ws.h_flag_accum);
+      ctx->launches++;
+      return 0;
+    }
+    DVO_CUDA(ctx, cudaMemcpyAsync(&ws.h_active[level_flag_slot(launch)], flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+    return 0;
+  };
 
-  for (int i = 0; i < 8; ++i) ws.h_active[i] = 0;
   if (max_log > 0) DVO_CUDA(ctx, cudaMemsetAsync(ws.d_iter_log, 0, sizeof(dvo_b200_iteration_stats) * (size_t)n * max_log, st));
   LevelLaunch lps[kMaxLevels][kMaxLevels];
   const PairLevel* d_pls[kMaxLevels];
@@ -1118,16 +1176,15 @@ int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dv
       seg_pls[sgi] = d_pls[gi];
     }
     int* flag = nullptr;
-    if ((rc = launch_segments(ctx, nseg, seg_lps, segs, seg_hmax, seg_pls, have_init ? ws.d_tinit : nullptr, n, max_log, nullptr, 0, 0, &flag)))
+    if ((rc = launch_segments(ctx, nseg, seg_lps, segs, seg_hmax, seg_pls, d_tinit, n, max_log, nullptr, 0, 0, &flag)))
       return rc;
-    DVO_CUDA(ctx, cudaMemcpyAsync(&ws.h_active[level_flag_slot(0)], flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+    if ((rc = keep_flag(0, flag))) return rc;
   } else {
     for (int gi = 0; gi < nlaunch; ++gi) {
       int* flag = nullptr;
-      if ((rc = launch_segments(ctx, 1, lps + gi, groups + gi, hmaxs + gi, d_pls + gi, have_init ? ws.d_tinit : nullptr, n, max_log,
-                                nullptr, 0, gi, &flag)))
+      if ((rc = launch_segments(ctx, 1, lps + gi, groups + gi, hmaxs + gi, d_pls + gi, d_tinit, n, max_log, nullptr, 0, gi, &flag)))
         return rc;
-      DVO_CUDA(ctx, cudaMemcpyAsync(&ws.h_active[level_flag_slot(gi)], flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+      if ((rc = keep_flag(gi, flag))) return rc;
     }
   }
   // results
@@ -1143,7 +1200,7 @@ int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dv
     ctx->launches++;
   }
   DVO_CUDA(ctx, cudaGetLastError());
-  ctx->pending_level_flags = nlaunch;   // checked at the next synchronisation point (device-results variant)
+  if (!enqueue) ctx->pending_level_flags = nlaunch;   // checked at the next synchronisation point (device-results variant)
   if (h_results) {
     size_t bytes = sizeof(dvo_b200_result) * n;
     if (bytes > ctx->h_results_bytes) {
@@ -1167,20 +1224,40 @@ int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dv
 }
 
 // The persistent kernels report a barrier / transaction timeout through a flag copied to pinned memory after every level.
-// Call after the stream has been synchronised.
-int check_level_flags(dvo_b200_ctx* ctx) {
+// fold_level_flags moves a reported code of the pending levels into the accumulated word, so that a call which reuses the
+// per-level slots does not lose it; check_level_flags reports (and clears) the accumulated code.  Both run after the
+// stream has been synchronised.
+void fold_level_flags(dvo_b200_ctx* ctx) {
   Workspace& ws = ctx->ws;
   const int nl = ctx->pending_level_flags;
   ctx->pending_level_flags = 0;
-  if (!ws.h_active) return 0;
+  if (!ws.h_active) return;
   for (int li = 0; li < nl && li < 8; ++li)
     if (ws.h_active[li] != 0) {
-      const int code = ws.h_active[li];
+      if (ws.h_flag_accum && *ws.h_flag_accum == 0) *ws.h_flag_accum = ws.h_active[li];
       ws.h_active[li] = 0;
-      return set_error(ctx, DVO_B200_ERR_CUDA, code == 2 ? "persistent level kernel: bulk-copy transaction timed out"
-                                                         : "persistent level kernel: squad barrier timed out");
     }
-  return 0;
+}
+
+int check_level_flags(dvo_b200_ctx* ctx) {
+  Workspace& ws = ctx->ws;
+  fold_level_flags(ctx);
+  if (!ws.h_flag_accum || *ws.h_flag_accum == 0) return 0;
+  const int code = *ws.h_flag_accum;
+  *ws.h_flag_accum = 0;
+  return set_error(ctx, DVO_B200_ERR_CUDA, code == 2 ? "persistent level kernel: bulk-copy transaction timed out"
+                                                     : "persistent level kernel: squad barrier timed out");
+}
+
+void tracker_release(dvo_b200_ctx* ctx) {
+  for (int i = 0; i < dvo_b200_ctx::kDescSlots; ++i) {
+    if (ctx->h_desc[i]) cudaFreeHost(ctx->h_desc[i]);
+    if (ctx->desc_staged[i]) cudaEventDestroy(ctx->desc_staged[i]);
+    ctx->h_desc[i] = nullptr; ctx->desc_staged[i] = nullptr;
+  }
+  ctx->desc_slot_bytes = 0;
+  if (ctx->ws.h_flag_accum) cudaFreeHost(ctx->ws.h_flag_accum);
+  ctx->ws.h_flag_accum = nullptr;
 }
 
 // Test hooks (dvo_b200_residual_image, dvo_b200_linearize): ONE Gauss-Newton iteration of the level kernel for one
@@ -1219,6 +1296,7 @@ int tracker_linearize(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, dvo_b200_py
   fill_pair_levels((PairLevel*)ctx->h_stage, 1, refs, curs, level);
   DVO_CUDA(ctx, cudaMemcpyAsync(ws.d_pair_level, ctx->h_stage, sizeof(PairLevel), cudaMemcpyHostToDevice, st));
   DVO_CUDA(ctx, cudaStreamSynchronize(st));
+  fold_level_flags(ctx);
   std::memcpy(ctx->h_stage, T, sizeof(double) * 16);
   float pp[4] = {0, 0, 0, 0};
   if (use_weights && prev_precision) std::memcpy(pp, prev_precision, sizeof(pp));

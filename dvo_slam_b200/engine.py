@@ -29,7 +29,11 @@ ABI_SYMBOLS = [
     "dvo_b200_profile_read", "dvo_b200_pyramid_device", "dvo_b200_sharded_create", "dvo_b200_sharded_destroy",
     "dvo_b200_sharded_num_shards", "dvo_b200_sharded_ctx", "dvo_b200_sharded_last_error", "dvo_b200_shard_range",
     "dvo_b200_sharded_pyramid_create_batch", "dvo_b200_sharded_pyramid_create_raw_batch", "dvo_b200_match_batch_sharded",
+    "dvo_b200_pyramid_create_device_batch", "dvo_b200_match_batch_enqueue",
 ]
+
+# dvo_b200_frame_format
+FRAME_F32, FRAME_GREY8_RAW16, FRAME_BGR8_RAW16 = 0, 1, 2
 
 
 class Config(C.Structure):
@@ -65,6 +69,63 @@ class LevelStats(C.Structure):
 class CResult(C.Structure):
     _fields_ = [("transformation", C.c_double * 16), ("information", C.c_double * 36), ("log_likelihood", C.c_double),
                 ("num_levels", C.c_int32), ("num_iterations_total", C.c_int32), ("levels", LevelStats * MAX_LEVELS)]
+
+
+class DeviceFrames(C.Structure):
+    """dvo_b200_device_frames: n images in device memory, strides in bytes."""
+    _fields_ = [("format", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("reserved", C.c_int32),
+                ("colour", C.c_void_p), ("colour_row_bytes", C.c_int64), ("colour_image_bytes", C.c_int64),
+                ("depth", C.c_void_p), ("depth_row_bytes", C.c_int64), ("depth_image_bytes", C.c_int64),
+                ("depth_scale", C.c_float)]
+
+
+def device_frames(colour, depth, depth_scale=None) -> DeviceFrames:
+    """dvo_b200_device_frames describing two torch tensors in place (no copy).
+
+    colour: [n,h,w] float32 (intensity) or uint8 (grey), or [n,h,w,3] uint8 (interleaved BGR); depth: [n,h,w] float32
+    (metres, NaN = invalid) with float32 colour, else 16-bit raw depth (torch.uint16, or int16 holding the same bits) and
+    depth_scale.  Unit stride is required along the pixels of a row; element strides become byte strides."""
+    import torch
+    u16 = tuple(t for t in (getattr(torch, "uint16", None), torch.int16) if t is not None)
+    if colour.dtype == torch.float32:
+        fmt = FRAME_F32
+        if depth.dtype != torch.float32:
+            raise ValueError("float32 colour takes float32 depth in metres")
+    elif colour.dtype == torch.uint8:
+        fmt = FRAME_BGR8_RAW16 if colour.dim() == 4 else FRAME_GREY8_RAW16
+        if depth.dtype not in u16:
+            raise ValueError("8-bit colour takes 16-bit raw depth (torch.uint16 or int16)")
+        if depth_scale is None:
+            raise ValueError("16-bit raw depth needs depth_scale")
+    else:
+        raise ValueError(f"colour dtype {colour.dtype}: float32, or uint8 grey / BGR")
+    if depth.dim() != 3 or colour.dim() != (4 if fmt == FRAME_BGR8_RAW16 else 3) or tuple(colour.shape[:3]) != tuple(depth.shape):
+        raise ValueError(f"shapes {tuple(colour.shape)} / {tuple(depth.shape)}: colour [n,h,w] or [n,h,w,3], depth [n,h,w]")
+    if fmt == FRAME_BGR8_RAW16 and (colour.shape[3] != 3 or colour.stride(3) != 1 or colour.stride(2) != 3):
+        raise ValueError("BGR colour needs 3 interleaved channels with unit stride, pixels 3 bytes apart")
+    if fmt != FRAME_BGR8_RAW16 and colour.stride(2) != 1:
+        raise ValueError("colour needs unit stride along a row")
+    if depth.stride(2) != 1:
+        raise ValueError("depth needs unit stride along a row")
+    n, h, w = depth.shape
+
+    def strides(t):
+        row = t.stride(1) * t.element_size()
+        return row, (t.stride(0) * t.element_size() if n > 1 else h * row)
+
+    f = DeviceFrames()
+    f.format, f.width, f.height, f.reserved = fmt, w, h, 0
+    f.colour, (f.colour_row_bytes, f.colour_image_bytes) = colour.data_ptr(), strides(colour)
+    f.depth, (f.depth_row_bytes, f.depth_image_bytes) = depth.data_ptr(), strides(depth)
+    f.depth_scale = float(depth_scale) if depth_scale is not None else 0.0
+    return f
+
+
+def result_transformations(records):
+    """[n, 4, 4] float64 view (no copy) of Result.Transformation in a uint8 tensor of n dvo_b200_result records, as
+    Engine.match_batch_enqueue returns it: transformation is the first field of the record."""
+    import torch
+    return records.view(torch.float64)[:, :16].view(records.shape[0], 4, 4)
 
 
 class Result:
@@ -121,6 +182,9 @@ def load_library():
     L.dvo_b200_pyramid_create_raw_batch.argtypes = [vp, i32, vp, vp, C.c_float, i32, i32, C.c_float, C.c_float, C.c_float, C.c_float, i32, C.POINTER(vp)]
     L.dvo_b200_pyramid_create_bgr_batch.argtypes = [vp, i32, vp, vp, C.c_float, i32, i32, C.c_float, C.c_float, C.c_float, C.c_float, i32, C.POINTER(vp)]
     L.dvo_b200_pyramid_device.argtypes = [vp]
+    L.dvo_b200_pyramid_create_device_batch.argtypes = [vp, i32, C.POINTER(DeviceFrames), C.c_float, C.c_float, C.c_float, C.c_float, i32,
+                                                       C.POINTER(vp)]
+    L.dvo_b200_match_batch_enqueue.argtypes = [vp, C.POINTER(Config), i32, C.POINTER(vp), C.POINTER(vp), vp, vp]
     L.dvo_b200_sharded_create.argtypes = [i32, C.POINTER(i32), C.POINTER(vp)]
     L.dvo_b200_sharded_destroy.argtypes = [vp]
     L.dvo_b200_sharded_num_shards.argtypes = [vp]
@@ -343,6 +407,68 @@ class Engine:
         self._check(self.lib.dvo_b200_match_batch_device(self.ctx, C.byref(cfg), n, rh, ch,
                                                          T.ctypes.data_as(C.POINTER(C.c_double)) if T is not None else None,
                                                          C.c_void_p(d_results_ptr)))
+
+    # ---- frames and results in GPU memory (torch tensors) ----
+    def _torch_stream(self):
+        """The context's stream as a torch stream (for ordering against torch work)."""
+        import torch
+        if getattr(self, "_ext_stream", None) is None:
+            self._ext_stream = torch.cuda.ExternalStream(self.stream, device=torch.device("cuda", self.device))
+        return self._ext_stream
+
+    def _check_on_device(self, t, name):
+        if not t.is_cuda or t.device.index != self.device:
+            raise ValueError(f"{name} must be a CUDA tensor on cuda:{self.device} (got {t.device})")
+
+    def pyramid_from_tensors(self, colour, depth, intrinsics, levels: int, depth_scale=None) -> list[Pyramid]:
+        """Pyramids of n frames already in GPU memory, read in place (dvo_b200_pyramid_create_device_batch).
+
+        colour: [n,h,w] float32 or uint8, or [n,h,w,3] uint8 BGR; depth: [n,h,w] float32 metres, or 16-bit raw depth
+        (torch.uint16 / int16) with depth_scale.  Any row / image strides with unit stride along a row.  The context's stream
+        waits for the work already queued on the current torch stream, and the inputs are marked as used on the context's
+        stream, so the caching allocator does not reuse their memory before the build has read them.  Equal bit for bit to
+        the host entry point of the same format on the same pixels."""
+        import torch
+        self._check_on_device(colour, "colour")
+        self._check_on_device(depth, "depth")
+        frames = device_frames(colour, depth, depth_scale)
+        n = depth.shape[0]
+        ext = self._torch_stream()
+        ext.wait_stream(torch.cuda.current_stream(colour.device))
+        fx, fy, ox, oy = intrinsics
+        out = (C.c_void_p * n)()
+        self._check(self.lib.dvo_b200_pyramid_create_device_batch(self.ctx, n, C.byref(frames), fx, fy, ox, oy, levels, out))
+        colour.record_stream(ext)
+        depth.record_stream(ext)
+        return [Pyramid(self, out[i]) for i in range(n)]
+
+    def match_batch_enqueue(self, refs, curs, cfg: Config, T_init=None):
+        """dvo_b200_match_batch_enqueue: returns a uint8 CUDA tensor [n, sizeof(dvo_b200_result)] of result records,
+        ordered onto the current torch stream; the host does not wait for the GPU.  T_init: CUDA float64 [n,4,4]
+        (Result.Transformation on entry, read iff cfg.use_initial_estimate).  result_transformations() views the poses."""
+        import torch
+        n = len(refs)
+        assert n == len(curs) and n > 0
+        dev = torch.device("cuda", self.device)
+        cur = torch.cuda.current_stream(dev)
+        T = None
+        if T_init is not None:
+            self._check_on_device(T_init, "T_init")
+            if T_init.dtype != torch.float64 or tuple(T_init.shape) != (n, 4, 4):
+                raise ValueError(f"T_init: float64 [{n},4,4] expected, got {T_init.dtype} {tuple(T_init.shape)}")
+            T = T_init.contiguous()
+        records = torch.empty((n, C.sizeof(CResult)), dtype=torch.uint8, device=dev)
+        rh = (C.c_void_p * n)(*[p.handle for p in refs])
+        ch = (C.c_void_p * n)(*[p.handle for p in curs])
+        ext = self._torch_stream()
+        ext.wait_stream(cur)
+        self._check(self.lib.dvo_b200_match_batch_enqueue(self.ctx, C.byref(cfg), n, rh, ch, T.data_ptr() if T is not None else None,
+                                                          records.data_ptr()))
+        records.record_stream(ext)
+        if T is not None:
+            T.record_stream(ext)
+        cur.wait_stream(ext)
+        return records
 
     def residual_image(self, ref: Pyramid, cur: Pyramid, level: int, T, cfg: Config | None = None):
         cfg = cfg or Config()

@@ -139,6 +139,36 @@ int dvo_b200_pyramid_create_raw_batch(dvo_b200_ctx* ctx, int32_t n, const uint8_
 int dvo_b200_pyramid_create_bgr_batch(dvo_b200_ctx* ctx, int32_t n, const uint8_t* bgr, const uint16_t* raw_depth,
                                       float depth_scale, int32_t width, int32_t height, float fx, float fy, float ox,
                                       float oy, int32_t levels, dvo_b200_pyramid** out /* n handles */);
+/* ---- frames already in GPU memory ---------------------------------------------------------------------------------
+ * The three pixel formats of the host entry points above, read in place from DEVICE memory (a decoder surface, a
+ * rendered frame, a tensor): the pyramids equal bit for bit those the matching host entry point builds from the same
+ * pixels (dvo_b200_pyramid_create_batch / _raw_batch / _bgr_batch). */
+typedef enum dvo_b200_frame_format {
+  DVO_B200_FRAME_F32 = 0,          /* float32 intensity (0..255 units) + float32 depth in metres, NaN = invalid */
+  DVO_B200_FRAME_GREY8_RAW16 = 1,  /* 8-bit grey + 16-bit raw depth: depth = raw * depth_scale, 0 -> NaN       */
+  DVO_B200_FRAME_BGR8_RAW16 = 2    /* interleaved 8-bit BGR (OpenCV order) + 16-bit raw depth                  */
+} dvo_b200_frame_format;
+
+/* n images of width x height.  Pixel (x, y) of image i of the colour plane lies at
+ *   colour + i * colour_image_bytes + y * colour_row_bytes + x * (4 bytes F32, 1 GREY8, 3 BGR8)
+ * and likewise for depth (4 bytes F32, 2 RAW16): pitched buffers, slices of wider tensors and every k-th image of a batch
+ * need no copy.  Row strides are at least width x pixel size, image strides (read only for n > 1) at least height x row
+ * stride; pointers and strides are multiples of the element size (4 for float32, 2 for 16-bit). */
+typedef struct dvo_b200_device_frames {
+  int32_t format, width, height, reserved;                             /* dvo_b200_frame_format; reserved = 0 */
+  const void* colour;  int64_t colour_row_bytes, colour_image_bytes;   /* DEVICE pointer to image 0 + strides in bytes */
+  const void* depth;   int64_t depth_row_bytes,  depth_image_bytes;
+  float depth_scale;                                                   /* raw formats only */
+} dvo_b200_device_frames;
+
+/* Both pointers must be device (or managed) memory of the context's device; host memory is refused with
+ * DVO_B200_ERR_INVALID_ARGUMENT and nothing is copied.  The frames are read on the context's stream: a caller that writes
+ * them on another stream makes the context's stream wait for that work first (cudaStreamWaitEvent).  The pyramids keep no
+ * reference to the frames, so work enqueued later on the context's stream may overwrite them.  Moves no frame over the bus
+ * and does not synchronise. */
+int dvo_b200_pyramid_create_device_batch(dvo_b200_ctx* ctx, int32_t n, const dvo_b200_device_frames* frames,
+                                         float fx, float fy, float ox, float oy, int32_t levels, dvo_b200_pyramid** out);
+
 int dvo_b200_pyramid_device(const dvo_b200_pyramid* p);   /* CUDA ordinal the pyramid lives on (-1: null handle) */
 int dvo_b200_pyramid_retain(dvo_b200_pyramid* p);   /* boost::shared_ptr semantics of RgbdImagePyramidPtr */
 int dvo_b200_pyramid_release(dvo_b200_pyramid* p);
@@ -174,6 +204,17 @@ int dvo_b200_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int32_t 
 int dvo_b200_match_batch_device(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int32_t n,
                                 dvo_b200_pyramid* const* references, dvo_b200_pyramid* const* currents,
                                 const double* T_init, void* d_results);
+
+/* Enqueue-only batch alignment: d_T_init (DEVICE, n*16 doubles, row-major Result.Transformation on entry, read iff
+ * cfg->use_initial_estimate; may be NULL) and d_results (DEVICE, n dvo_b200_result) live on the context's device and are
+ * read / written on its stream, so steps can be chained on a stream without the host waiting.  Once the context is warm
+ * (an earlier call with at least as many pairs and levels), the call does not block on the GPU: the pair descriptors --
+ * the only host-to-device traffic -- go up through a ring of pinned slots, and the host waits only when the ring wraps
+ * onto a slot the GPU has not read yet.  A kernel timeout in any call enqueued since the last synchronisation is
+ * reported by the next dvo_b200_synchronize.  Pyramids built by another context must stay referenced until then. */
+int dvo_b200_match_batch_enqueue(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int32_t n,
+                                 dvo_b200_pyramid* const* references, dvo_b200_pyramid* const* currents,
+                                 const double* d_T_init, void* d_results);
 
 /* ---- one process, several GPUs (SURVEY.md 8e) ----------------------------------------------------
  * The reference's batch producers are single-process C++ loops over independent match() calls
