@@ -107,6 +107,18 @@ int check_plane(dvo_b200_ctx* ctx, const char* name, const void* p, int64_t row_
   return check_device_pointer(ctx, p, f);
 }
 
+// device result records and initial estimates of the enqueue entry points
+int check_enqueue_buffers(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, const double* d_T_init, void* d_results, const std::string& f) {
+  if ((uintptr_t)d_results % 8) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + ": d_results is not 8-byte aligned");
+  int rc = check_device_pointer(ctx, d_results, f + ": d_results");
+  if (rc) return rc;
+  if (cfg && cfg->use_initial_estimate && d_T_init) {
+    if ((uintptr_t)d_T_init % 8) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + ": d_T_init is not 8-byte aligned");
+    if ((rc = check_device_pointer(ctx, d_T_init, f + ": d_T_init"))) return rc;
+  }
+  return 0;
+}
+
 }  // namespace
 }  // namespace dvo_b200
 
@@ -396,14 +408,124 @@ int dvo_b200_match_batch_enqueue(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, 
                                  dvo_b200_pyramid* const* currents, const double* d_T_init, void* d_results) {
   if (!ctx || !d_results) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_enqueue: null argument");
   cudaSetDevice(ctx->device);
-  if ((uintptr_t)d_results % 8) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_enqueue: d_results is not 8-byte aligned");
-  int rc = check_device_pointer(ctx, d_results, "match_batch_enqueue: d_results");
+  int rc = check_enqueue_buffers(ctx, cfg, d_T_init, d_results, "match_batch_enqueue");
   if (rc) return rc;
-  if (cfg && cfg->use_initial_estimate && d_T_init) {
-    if ((uintptr_t)d_T_init % 8) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_enqueue: d_T_init is not 8-byte aligned");
-    if ((rc = check_device_pointer(ctx, d_T_init, "match_batch_enqueue: d_T_init"))) return rc;
-  }
   return tracker_match_batch(ctx, cfg, n, references, currents, d_T_init, nullptr, d_results, nullptr, 0, true);
+}
+
+int dvo_b200_selection_create(dvo_b200_ctx* ctx, dvo_b200_pyramid* p, int32_t predicate, float ti, float td,
+                              const uint8_t* const* level_masks, dvo_b200_selection** out) {
+  if (!ctx || !p || !out) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "selection_create: null argument");
+  if (predicate < DVO_B200_PREDICATE_GRADIENT_THRESHOLD || predicate > DVO_B200_PREDICATE_MASK_ONLY)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "selection_create: predicate " + std::to_string(predicate) + " is unknown");
+  if (p->device != ctx->device) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "selection_create: pyramid lives on another device");
+  cudaSetDevice(ctx->device);
+  SelMaskInput mi;
+  if (level_masks)
+    for (int l = 0; l < p->levels; ++l) mi.per_level[l] = level_masks[l];
+  dvo_b200_pyramid* pyrs[1] = {p};
+  return selection_build_batch(ctx, 1, pyrs, predicate, ti, td, mi, out);
+}
+
+int dvo_b200_selection_create_device_batch(dvo_b200_ctx* ctx, int32_t n, dvo_b200_pyramid* const* pyramids, int32_t predicate,
+                                           float ti, float td, const void* d_masks, int64_t row_bytes, int64_t image_bytes,
+                                           dvo_b200_selection** out) {
+  const char* f = "selection_create_device_batch: ";
+  if (!ctx || !pyramids || !out || n <= 0) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, std::string(f) + "null/invalid argument");
+  if (predicate < DVO_B200_PREDICATE_GRADIENT_THRESHOLD || predicate > DVO_B200_PREDICATE_MASK_ONLY)
+    return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + std::string("predicate ") + std::to_string(predicate) + " is unknown");
+  for (int i = 0; i < n; ++i) {
+    const dvo_b200_pyramid* p = pyramids[i];
+    if (!p) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, std::string(f) + "null pyramid");
+    if (p->device != ctx->device) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, std::string(f) + "pyramid lives on another device");
+    if (p->levels != pyramids[0]->levels || p->L[0].w != pyramids[0]->L[0].w || p->L[0].h != pyramids[0]->L[0].h)
+      return set_error(ctx, DVO_B200_ERR_SHAPE_MISMATCH, std::string(f) + "all pyramids must share width, height and levels");
+  }
+  cudaSetDevice(ctx->device);
+  SelMaskInput mi;
+  if (d_masks) {
+    const int w = pyramids[0]->L[0].w, h = pyramids[0]->L[0].h;
+    if (row_bytes < w)
+      return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + std::string("row_bytes ") + std::to_string(row_bytes) + " < width");
+    if (n > 1 && image_bytes < (int64_t)h * row_bytes)
+      return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, f + std::string("image_bytes ") + std::to_string(image_bytes) + " < height x row_bytes");
+    int rc = check_device_pointer(ctx, d_masks, std::string(f) + "d_masks");
+    if (rc) return rc;
+    mi.level0 = (const uint8_t*)d_masks; mi.row = (size_t)row_bytes; mi.img = n > 1 ? (size_t)image_bytes : 0;
+  }
+  return selection_build_batch(ctx, n, pyramids, predicate, ti, td, mi, out);
+}
+
+int dvo_b200_selection_retain(dvo_b200_selection* s) {
+  if (!s) return DVO_B200_ERR_INVALID_ARGUMENT;
+  s->refcount.fetch_add(1, std::memory_order_relaxed);
+  return 0;
+}
+
+int dvo_b200_selection_release(dvo_b200_selection* s) {
+  if (!s) return DVO_B200_ERR_INVALID_ARGUMENT;
+  // as dvo_b200_pyramid_release: the slab returns to the building ctx's pool and is rewritten only by work enqueued later
+  // on that ctx's stream
+  if (s->refcount.fetch_sub(1, std::memory_order_acq_rel) == 1) selection_free(s);
+  return 0;
+}
+
+dvo_b200_pyramid* dvo_b200_selection_pyramid(dvo_b200_selection* s) { return s ? s->pyr : nullptr; }
+
+int dvo_b200_selection_download(dvo_b200_ctx* ctx, const dvo_b200_selection* s, int32_t level, int64_t* count, uint8_t* mask) {
+  if (!s || level < 0 || level >= s->pyr->levels) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "selection_download: invalid argument");
+  cudaSetDevice(s->device);
+  const LevelInfo& L = s->pyr->L[level];
+  if (ctx) DVO_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  if (s->slab && s->slab->ready) DVO_CUDA(ctx, cudaEventSynchronize(s->slab->ready));   // the selection's build has finished
+  int info[2];
+  DVO_CUDA(ctx, cudaMemcpy(info, s->sel_info + 2 * level, sizeof(info), cudaMemcpyDeviceToHost));
+  if (count) *count = info[0];
+  if (mask) {
+    std::vector<uint32_t> words(L.words);
+    DVO_CUDA(ctx, cudaMemcpy(words.data(), s->mask + L.mask_off, sizeof(uint32_t) * L.words, cudaMemcpyDeviceToHost));
+    for (int i = 0; i < L.n; ++i) mask[i] = (words[i >> 5] >> (i & 31)) & 1u;
+  }
+  if (ctx) ctx->d2h_bytes += sizeof(info) + (mask ? sizeof(uint32_t) * L.words : 0);
+  return 0;
+}
+
+}  // extern "C"
+
+// the pyramids of n selections, for the shared match path
+static int selection_refs(dvo_b200_ctx* ctx, int n, dvo_b200_selection* const* sels, std::vector<dvo_b200_pyramid*>& refs) {
+  if (!sels || n <= 0) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_selected: null argument");
+  refs.resize(n);
+  for (int i = 0; i < n; ++i) {
+    if (!sels[i]) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_selected: null selection");
+    refs[i] = sels[i]->pyr;
+  }
+  return 0;
+}
+
+extern "C" {
+
+int dvo_b200_match_batch_selected(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int32_t n, dvo_b200_selection* const* references,
+                                  dvo_b200_pyramid* const* currents, const double* T_init, dvo_b200_result* results,
+                                  dvo_b200_iteration_stats* iteration_stats, int32_t max_iteration_stats) {
+  if (!ctx || !results) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_selected: null argument");
+  cudaSetDevice(ctx->device);
+  std::vector<dvo_b200_pyramid*> refs;
+  int rc = selection_refs(ctx, n, references, refs);
+  if (rc) return rc;
+  return tracker_match_batch(ctx, cfg, n, refs.data(), currents, T_init, results, nullptr, iteration_stats,
+                             iteration_stats ? max_iteration_stats : 0, false, references);
+}
+
+int dvo_b200_match_batch_selected_enqueue(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int32_t n, dvo_b200_selection* const* references,
+                                          dvo_b200_pyramid* const* currents, const double* d_T_init, void* d_results) {
+  if (!ctx || !d_results) return set_error(ctx, DVO_B200_ERR_INVALID_ARGUMENT, "match_batch_selected_enqueue: null argument");
+  cudaSetDevice(ctx->device);
+  int rc = check_enqueue_buffers(ctx, cfg, d_T_init, d_results, "match_batch_selected_enqueue");
+  if (rc) return rc;
+  std::vector<dvo_b200_pyramid*> refs;
+  if ((rc = selection_refs(ctx, n, references, refs))) return rc;
+  return tracker_match_batch(ctx, cfg, n, refs.data(), currents, d_T_init, nullptr, d_results, nullptr, 0, true, references);
 }
 
 int dvo_b200_residual_image(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, dvo_b200_pyramid* reference,

@@ -109,6 +109,24 @@ struct dvo_b200_pyramid {
   uint64_t id = 0;
 };
 
+// A reference point selection of one pyramid (dvo::core::PointSelection with its own predicate and an optional per-pixel
+// mask), separate from the pyramid's built-in selection: its own copy of the reference tile records of every level (only
+// the Zsel channel differs from the pyramid's), its own mask words and {S, last}.  The level kernel reads nothing else of
+// the selection, so an alignment against it runs the same kernel over the same bytes.  The template and the per-tile depth
+// ranges are borrowed from the pyramid, which the selection retains.
+struct dvo_b200_selection {
+  int device = 0;
+  std::atomic<int> refcount{1};
+  dvo_b200_pyramid* pyr = nullptr;   // retained
+  dvo_b200::Slab* slab = nullptr;    // shared by the selections of one build; slab->ready = build finished
+  float2* rec = nullptr;             // device: tile records of every level (rec_off[l] float2 into it)
+  uint32_t* mask = nullptr;          // device: mask words of every level, at the pyramid's mask_off
+  int* sel_info = nullptr;           // device: per level {S, last selected linear pixel index}
+  size_t rec_off[dvo_b200::kMaxLevels] = {};
+  int predicate = 0;
+  float ti = 0.f, td = 0.f;
+};
+
 namespace dvo_b200 {
 
 // ---- per-pair device state ---------------------------------------------------------------------
@@ -250,6 +268,16 @@ int pyramid_build_batch_input(dvo_b200_ctx* ctx, int n, const FrameInput& in, in
                               int levels, float ti, float td, dvo_b200_pyramid** out);
 int pyramid_reselect(dvo_b200_ctx* ctx, dvo_b200_pyramid* p, float ti, float td);
 void pyramid_free(dvo_b200_pyramid* p);
+// Selection masks of a build: level-0 masks read at byte strides and subsampled (shift = level, the depth chain), or one
+// host-staged mask per level (dense rows, shift 0; a null level allows every pixel).  mask == null everywhere: no mask.
+struct SelMaskInput {
+  const uint8_t* level0 = nullptr; size_t row = 0, img = 0;   // device level-0 masks of n images
+  const uint8_t* per_level[kMaxLevels] = {};                  // n == 1: dense h_l x w_l bytes per level, or null
+};
+// n selections of n pyramids with identical geometry, one slab; out[i] retains pyrs[i].
+int selection_build_batch(dvo_b200_ctx* ctx, int n, dvo_b200_pyramid* const* pyrs, int predicate, float ti, float td,
+                          const SelMaskInput& masks, dvo_b200_selection** out);
+void selection_free(dvo_b200_selection* s);
 void pool_close(dvo_b200_ctx* ctx);
 int ensure_stage(dvo_b200_ctx* ctx, size_t dev_bytes, size_t host_bytes);
 
@@ -259,7 +287,10 @@ int ensure_stage(dvo_b200_ctx* ctx, size_t dev_bytes, size_t host_bytes);
 // device memory, the descriptors go through the slot ring and the host does not wait for the GPU.
 int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dvo_b200_pyramid* const* refs,
                         dvo_b200_pyramid* const* curs, const double* T_init, dvo_b200_result* h_results,
-                        void* d_results, dvo_b200_iteration_stats* iter_stats, int max_iter_stats, bool enqueue = false);
+                        void* d_results, dvo_b200_iteration_stats* iter_stats, int max_iter_stats, bool enqueue = false,
+                        dvo_b200_selection* const* sels = nullptr);
+// sels != null: pair i aligns against selection sels[i] of refs[i] (= sels[i]->pyr) instead of the pyramid's own selection,
+// and cfg's derivative thresholds are not read.
 int check_level_flags(dvo_b200_ctx* ctx);   // after a stream synchronisation: did a level kernel report a timeout?
 void fold_level_flags(dvo_b200_ctx* ctx);   // after a stream synchronisation: keep reported timeouts for check_level_flags
 void tracker_release(dvo_b200_ctx* ctx);    // frees the tracker's pinned buffers and events (stream synchronised)

@@ -5,6 +5,7 @@
 // default predicate (point_selection.cpp:89-152, point_selection.h:63-66).
 #include "common.cuh"
 
+#include <algorithm>
 #include <cstdio>
 #include <cstring>
 
@@ -248,6 +249,61 @@ __global__ void k_reselect(const float2* __restrict__ P0, float2* __restrict__ r
   if ((threadIdx.x & 31) == 0 && idx < ((n + 31) / 32) * 32) mask[idx >> 5] = m;
 }
 
+// One level of n point selections (blockIdx.y = selection), each over its own pyramid (src[img]: that pyramid's planes).
+// Per pixel: the predicate from the pyramid's P0 / P2 planes and the gradient rows of its records, AND the mask, then the
+// (I, Zsel) cell (Zsel = Z' where selected, NaN elsewhere, as k_reselect writes it), the gradient cell and the mask word
+// (ballot).  Threads below ntiles x kTileW also copy one tile column of what no pixel owns: the tx slice and the cells
+// outside the image.  The mask, if any, is read at m[img * m_img + (y << m_shift) * m_row + (x << m_shift)], nonzero =
+// allowed: m_shift = level subsamples a level-0 mask like the depth chain, m_shift = 0 reads a mask of this level.
+__global__ void __launch_bounds__(256)
+k_sel_build(const float2* const* __restrict__ src, size_t plane_off, size_t src_rec_off, int nbands, int ntiles, int w, int h,
+            int pitch, const uint8_t* __restrict__ m, size_t m_row, size_t m_img, int m_shift, float2* __restrict__ rec,
+            size_t rec_per_image, size_t rec_off, uint32_t* __restrict__ masks, size_t mask_words_per_image, size_t mask_off,
+            int words, int predicate, float ti, float td) {
+  const int img = blockIdx.y;
+  const int n = w * h;
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  const float2* P0 = src[img] + plane_off;
+  const float2* srec = src[img] + src_rec_off;
+  float2* drec = rec + img * rec_per_image + rec_off;
+  const float nanv = __int_as_float(0x7fc00000);
+  bool sel = false;
+  if (idx < n) {
+    const int y = idx / w, x = idx - y * w;
+    const size_t o = (size_t)y * pitch + x;
+    const float2* P2 = P0 + (size_t)pitch * h;
+    const size_t rc = rec_cell(x, y, nbands);
+    const int xp = max(x - 1, 0), xn = min(x + 1, w - 1), yp = max(y - 1, 0), yn = min(y + 1, h - 1);
+    const float2 a = P0[o], g = srec[rc + kRecP1];
+    const float zx = (P2[(size_t)y * pitch + xn].y - P2[(size_t)y * pitch + xp].y) * 0.5f;
+    const float zy = (P2[(size_t)yn * pitch + x].y - P2[(size_t)yp * pitch + x].y) * 0.5f;
+    if (predicate == DVO_B200_PREDICATE_GRADIENT_THRESHOLD)   // ValidPointAndGradientThresholdPredicate (point_selection.h:52-67)
+      sel = !is_nan(a.y) && (fabsf(g.x) > ti || fabsf(g.y) > ti || fabsf(zx) > td || fabsf(zy) > td);
+    else if (predicate == DVO_B200_PREDICATE_VALID_POINT)     // ValidPointPredicate (point_selection.h:39-47): true depth
+      sel = !is_nan(P2[o].y) && !is_nan(zx) && !is_nan(zy);
+    else                                                      // MASK_ONLY
+      sel = true;
+    if (m) sel = sel && __ldg(m + img * m_img + (size_t)(y << m_shift) * m_row + ((size_t)x << m_shift)) != 0;
+    drec[rc] = make_float2(a.x, sel ? a.y : nanv);
+    drec[rc + kRecP1] = g;
+  }
+  const unsigned bits = __ballot_sync(0xffffffffu, sel);
+  if ((threadIdx.x & 31) == 0 && idx < words * 32) masks[img * mask_words_per_image + mask_off + (idx >> 5)] = bits;
+  if (idx < ntiles * kTileW) {
+    const int tile = idx / kTileW, cx = idx - tile * kTileW;
+    const int s = tile / nbands, b = tile - s * nbands;
+    const int x = b * kTileW + cx, y0 = s * kTileH;
+    const float2* st = srec + (size_t)tile * kRecF2;
+    float2* dt = drec + (size_t)tile * kRecF2;
+    reinterpret_cast<float*>(dt + kRecTx)[cx] = reinterpret_cast<const float*>(st + kRecTx)[cx];
+    const int r0 = x >= w ? 0 : min(max(h - y0, 0), kTileH);
+    for (int r = r0; r < kTileH; ++r) {
+      dt[r * kTileW + cx] = st[r * kTileW + cx];
+      dt[kRecP1 + r * kTileW + cx] = st[kRecP1 + r * kTileW + cx];
+    }
+  }
+}
+
 // point-cloud template tx[x] = (x - ox)/fx, ty[y] = (y - oy)/fy (IEEE division, rgbd_image.cpp:197-198)
 __global__ void k_template(float* __restrict__ tmpl, size_t tmpl_per_image, size_t off, int w, int h, float fx,
                            float fy, float ox, float oy) {
@@ -305,10 +361,9 @@ static Slab* acquire_slab(dvo_b200_ctx* ctx, size_t bytes) {
   return s;
 }
 
-// Called from any host thread, possibly after the owning context has been destroyed.
-void pyramid_free(dvo_b200_pyramid* p) {
-  Slab* s = p->slab;
-  delete p;
+// Drops one reference to a slab: back to its context's pool, or freed if that context is gone.  Called from any host
+// thread, possibly after the owning context has been destroyed.
+static void slab_unref(Slab* s) {
   if (!s) return;
   std::shared_ptr<SlabPool> pool = s->pool;    // keeps the pool alive while its mutex is held
   std::lock_guard<std::mutex> lock(pool->mu);
@@ -316,6 +371,20 @@ void pyramid_free(dvo_b200_pyramid* p) {
     if (pool->closed) { cudaSetDevice(pool->device); destroy_slab(s); }
     else pool->free.insert({s->bytes, s});
   }
+}
+
+void pyramid_free(dvo_b200_pyramid* p) {
+  Slab* s = p->slab;
+  delete p;
+  slab_unref(s);
+}
+
+void selection_free(dvo_b200_selection* s) {
+  dvo_b200_pyramid* p = s->pyr;
+  Slab* slab = s->slab;
+  delete s;
+  slab_unref(slab);
+  if (p && p->refcount.fetch_sub(1, std::memory_order_acq_rel) == 1) pyramid_free(p);
 }
 
 // The context goes away: free what is pooled, and have slabs still referenced by live pyramids freed on release.
@@ -470,6 +539,95 @@ int pyramid_reselect(dvo_b200_ctx* ctx, dvo_b200_pyramid* p, float ti, float td)
   DVO_CUDA(ctx, cudaGetLastError());
   if (p->slab && p->slab->ready) DVO_CUDA(ctx, cudaEventRecord(p->slab->ready, st));
   p->sel_ti = ti; p->sel_td = td;
+  return 0;
+}
+
+// Layout of one selection inside its slab: the tile records of every level, then the mask words (at the pyramid's
+// mask_off), then {S, last} per level.  The only part that differs from the pyramid is the Zsel channel and the masks.
+int selection_build_batch(dvo_b200_ctx* ctx, int n, dvo_b200_pyramid* const* pyrs, int predicate, float ti, float td,
+                          const SelMaskInput& mi, dvo_b200_selection** out) {
+  const dvo_b200_pyramid* p0 = pyrs[0];
+  const int levels = p0->levels;
+  size_t rec_off[kMaxLevels], rec_f2 = 0;
+  for (int l = 0; l < levels; ++l) {
+    rec_off[l] = rec_f2;
+    rec_f2 += (size_t)p0->L[l].nbands * p0->L[l].nstrips * kRecF2;
+  }
+  rec_f2 = align_up(rec_f2, 32);
+  const size_t mask_words = align_up(p0->L[levels - 1].mask_off + p0->L[levels - 1].words, 64);
+  const int sel_ints = 2 * kMaxLevels;
+  const size_t bytes_rec = (size_t)n * rec_f2 * sizeof(float2);
+  const size_t bytes_mask = (size_t)n * mask_words * sizeof(uint32_t);
+  const size_t bytes_sel = align_up((size_t)n * sel_ints * sizeof(int), 256);
+  const size_t bytes_tab = (size_t)n * sizeof(const float2*);
+  Slab* slab = acquire_slab(ctx, bytes_rec + bytes_mask + bytes_sel + bytes_tab);
+  if (!slab) return set_error(ctx, DVO_B200_ERR_OUT_OF_MEMORY, "selection: cudaMalloc failed");
+  char* base = (char*)slab->base;
+  float2* rec = (float2*)base;
+  uint32_t* masks = (uint32_t*)(base + bytes_rec);
+  int* sel = (int*)(base + bytes_rec + bytes_mask);
+  const float2** tab = (const float2**)(base + bytes_rec + bytes_mask + bytes_sel);
+  cudaStream_t st = ctx->stream;
+
+  // host per-level masks go up through the device staging area (a pageable source is copied before the call returns)
+  const uint8_t* staged[kMaxLevels] = {};
+  size_t stage_bytes = 0, stage_off[kMaxLevels] = {};
+  for (int l = 0; l < levels; ++l)
+    if (mi.per_level[l]) { stage_off[l] = stage_bytes; stage_bytes += align_up((size_t)p0->L[l].n, 256); }
+  if (stage_bytes) {
+    int rc = ensure_stage(ctx, stage_bytes, 0);
+    if (rc) { slab->refs = 1; slab_unref(slab); return rc; }
+    for (int l = 0; l < levels; ++l)
+      if (mi.per_level[l]) {
+        staged[l] = (const uint8_t*)ctx->d_stage + stage_off[l];
+        DVO_CUDA(ctx, cudaMemcpyAsync((void*)staged[l], mi.per_level[l], (size_t)p0->L[l].n, cudaMemcpyHostToDevice, st));
+        ctx->h2d_bytes += p0->L[l].n;
+      }
+  }
+  std::vector<const float2*> h_tab(n);
+  for (int i = 0; i < n; ++i) {
+    h_tab[i] = pyrs[i]->planes;
+    // a pyramid built on another ctx's stream: order this stream after its build
+    if (pyrs[i]->slab && pyrs[i]->slab->pool != ctx->pool && pyrs[i]->slab->ready) cudaStreamWaitEvent(st, pyrs[i]->slab->ready, 0);
+  }
+  DVO_CUDA(ctx, cudaMemcpyAsync(tab, h_tab.data(), bytes_tab, cudaMemcpyHostToDevice, st));
+  ctx->h2d_bytes += bytes_tab;
+  {
+    ProfScope prof(ctx, 4, 3 * levels);
+    const int T = 256;
+    for (int l = 0; l < levels; ++l) {
+      const LevelInfo& q = p0->L[l];
+      const uint8_t* m = nullptr;
+      size_t m_row = 0, m_img = 0;
+      int m_shift = 0;
+      if (mi.level0) { m = mi.level0; m_row = mi.row; m_img = mi.img; m_shift = l; }
+      else if (staged[l]) { m = staged[l]; m_row = (size_t)q.w; }
+      const int ntiles = q.nbands * q.nstrips;
+      const int threads = std::max(q.words * 32, ntiles * kTileW);
+      k_sel_build<<<dim3((threads + T - 1) / T, n), T, 0, st>>>(tab, q.plane_off, q.rec_off, q.nbands, ntiles, q.w, q.h, q.pitch, m, m_row,
+                                                                  m_img, m_shift, rec, rec_f2, rec_off[l], masks, mask_words, q.mask_off,
+                                                                  q.words, predicate, ti, td);
+      k_sel_info<<<n, 32, 0, st>>>(masks, mask_words, q.mask_off, q.words, sel, sel_ints, l);
+      k_drop_odd_last<<<(n + 127) / 128, 128, 0, st>>>(rec, rec_f2, rec_off[l], q.nbands, q.w, sel, sel_ints, l, n);
+      ctx->launches += 3;
+    }
+  }
+  DVO_CUDA(ctx, cudaGetLastError());
+  if (!slab->ready) DVO_CUDA(ctx, cudaEventCreateWithFlags(&slab->ready, cudaEventDisableTiming));
+  DVO_CUDA(ctx, cudaEventRecord(slab->ready, st));
+  for (int i = 0; i < n; ++i) {
+    dvo_b200_selection* s = new dvo_b200_selection;
+    s->device = ctx->device;
+    s->pyr = pyrs[i];
+    pyrs[i]->refcount.fetch_add(1, std::memory_order_relaxed);
+    s->slab = slab; slab->refs++;
+    s->rec = rec + (size_t)i * rec_f2;
+    s->mask = masks + (size_t)i * mask_words;
+    s->sel_info = sel + (size_t)i * sel_ints;
+    std::memcpy(s->rec_off, rec_off, sizeof(size_t) * levels);
+    s->predicate = predicate; s->ti = ti; s->td = td;
+    out[i] = s;
+  }
   return 0;
 }
 

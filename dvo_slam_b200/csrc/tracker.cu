@@ -902,6 +902,20 @@ void fill_pair_levels(PairLevel* h, int n, dvo_b200_pyramid* const* refs, dvo_b2
   }
 }
 
+// The same descriptors against separate selections (refs[i] = sels[i]->pyr): tile records, mask and {S, last} come from
+// the selection, template and tile depth ranges from its pyramid.
+void fill_pair_levels_selected(PairLevel* h, int n, dvo_b200_pyramid* const* refs, dvo_b200_selection* const* sels,
+                               dvo_b200_pyramid* const* curs, int level) {
+  fill_pair_levels(h, n, refs, curs, level);
+  for (int i = 0; i < n; ++i) {
+    const dvo_b200_selection* s = sels[i];
+    PairLevel& q = h[i];
+    q.r0 = s->rec + s->rec_off[level]; q.r1 = q.r0;
+    q.rmask = s->mask + refs[i]->L[level].mask_off;
+    q.rsel = s->sel_info + 2 * level;
+  }
+}
+
 LevelLaunch make_level_launch(const LevelInfo& L, const dvo_b200_config* cfg, int li, int level) {
   LevelLaunch lp;
   lp.w = L.w; lp.h = L.h; lp.n = L.n; lp.pitch = L.pitch; lp.nbands = L.nbands; lp.nstrips = L.nstrips;
@@ -1030,9 +1044,13 @@ int acquire_desc_slot(dvo_b200_ctx* ctx, size_t bytes, int* slot) {
 
 int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dvo_b200_pyramid* const* refs,
                         dvo_b200_pyramid* const* curs, const double* T_init, dvo_b200_result* h_results,
-                        void* d_results_user, dvo_b200_iteration_stats* iter_stats, int max_iter_stats, bool enqueue) {
+                        void* d_results_user, dvo_b200_iteration_stats* iter_stats, int max_iter_stats, bool enqueue,
+                        dvo_b200_selection* const* sels) {
   int rc = check_batch(ctx, cfg, n, refs, curs);
   if (rc) return rc;
+  if (sels)   // a selection built on another ctx's stream: order this stream after its build
+    for (int i = 0; i < n; ++i)
+      if (sels[i]->slab && sels[i]->slab->pool != ctx->pool && sels[i]->slab->ready) cudaStreamWaitEvent(ctx->stream, sels[i]->slab->ready, 0);
   cudaStream_t st = ctx->stream;
   Workspace& ws = ctx->ws;
   const int last = cfg->last_level, first = cfg->first_level;
@@ -1104,8 +1122,10 @@ int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dv
   if (rc) return rc;
 
   // selection masks for non-default thresholds (PointSelection caches per pyramid, point_selection.cpp:100-113)
-  for (int i = 0; i < n; ++i)
-    if ((rc = pyramid_reselect(ctx, refs[i], cfg->intensity_derivative_threshold, cfg->depth_derivative_threshold))) return rc;
+  // (not for separate selections: their predicate decides, as in match(PointSelection&, ...), dense_tracking.cpp:131-135)
+  if (!sels)
+    for (int i = 0; i < n; ++i)
+      if ((rc = pyramid_reselect(ctx, refs[i], cfg->intensity_derivative_threshold, cfg->depth_derivative_threshold))) return rc;
 
   // Pair descriptors of every level and the initial estimates go into the pinned stage once; one small kernel copies
   // them to device memory (reads over PCIe: no H2D copy-engine work, no host round trip between the launches below).
@@ -1127,7 +1147,10 @@ int tracker_match_batch(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int n, dv
     h_desc = (PairLevel*)ctx->h_stage;
     if (have_init) std::memcpy((char*)ctx->h_stage + desc_bytes, T_init, init_bytes);
   }
-  for (int level = first, li = 0; level >= last; --level, ++li) fill_pair_levels(h_desc + (size_t)li * n, n, refs, curs, level);
+  for (int level = first, li = 0; level >= last; --level, ++li) {
+    if (sels) fill_pair_levels_selected(h_desc + (size_t)li * n, n, refs, sels, curs, level);
+    else fill_pair_levels(h_desc + (size_t)li * n, n, refs, curs, level);
+  }
   ctx->h2d_bytes += desc_bytes + init_bytes;
   {
     ProfScope prof(ctx, 2);

@@ -30,10 +30,23 @@ ABI_SYMBOLS = [
     "dvo_b200_sharded_num_shards", "dvo_b200_sharded_ctx", "dvo_b200_sharded_last_error", "dvo_b200_shard_range",
     "dvo_b200_sharded_pyramid_create_batch", "dvo_b200_sharded_pyramid_create_raw_batch", "dvo_b200_match_batch_sharded",
     "dvo_b200_pyramid_create_device_batch", "dvo_b200_match_batch_enqueue",
+    "dvo_b200_selection_create", "dvo_b200_selection_create_device_batch", "dvo_b200_selection_retain",
+    "dvo_b200_selection_release", "dvo_b200_selection_pyramid", "dvo_b200_selection_download",
+    "dvo_b200_match_batch_selected", "dvo_b200_match_batch_selected_enqueue",
 ]
 
 # dvo_b200_frame_format
 FRAME_F32, FRAME_GREY8_RAW16, FRAME_BGR8_RAW16 = 0, 1, 2
+# dvo_b200_predicate
+PREDICATE_GRADIENT_THRESHOLD, PREDICATE_VALID_POINT, PREDICATE_MASK_ONLY = 0, 1, 2
+
+
+def level_masks(mask0, levels: int):
+    """Per-level masks of a level-0 mask [h, w] by the subsample chain of the depth: M_l(y, x) = M_0(y << l, x << l) on the
+    (w >> l) x (h >> l) grid of level l.  What Engine.selections_from_tensors computes on the device."""
+    m = np.asarray(mask0)
+    h, w = m.shape
+    return [np.ascontiguousarray(m[::1 << l, ::1 << l][:h >> l, :w >> l] != 0).astype(np.uint8) for l in range(levels)]
 
 
 class Config(C.Structure):
@@ -185,6 +198,16 @@ def load_library():
     L.dvo_b200_pyramid_create_device_batch.argtypes = [vp, i32, C.POINTER(DeviceFrames), C.c_float, C.c_float, C.c_float, C.c_float, i32,
                                                        C.POINTER(vp)]
     L.dvo_b200_match_batch_enqueue.argtypes = [vp, C.POINTER(Config), i32, C.POINTER(vp), C.POINTER(vp), vp, vp]
+    L.dvo_b200_selection_create.argtypes = [vp, vp, i32, C.c_float, C.c_float, C.POINTER(C.c_void_p), C.POINTER(vp)]
+    L.dvo_b200_selection_create_device_batch.argtypes = [vp, i32, C.POINTER(vp), i32, C.c_float, C.c_float, vp, i64, i64, C.POINTER(vp)]
+    L.dvo_b200_selection_retain.argtypes = [vp]
+    L.dvo_b200_selection_release.argtypes = [vp]
+    L.dvo_b200_selection_pyramid.restype = vp
+    L.dvo_b200_selection_pyramid.argtypes = [vp]
+    L.dvo_b200_selection_download.argtypes = [vp, vp, i32, C.POINTER(i64), C.POINTER(C.c_uint8)]
+    L.dvo_b200_match_batch_selected.argtypes = [vp, C.POINTER(Config), i32, C.POINTER(vp), C.POINTER(vp), dp, C.POINTER(CResult),
+                                                C.POINTER(IterationStats), i32]
+    L.dvo_b200_match_batch_selected_enqueue.argtypes = [vp, C.POINTER(Config), i32, C.POINTER(vp), C.POINTER(vp), vp, vp]
     L.dvo_b200_sharded_create.argtypes = [i32, C.POINTER(i32), C.POINTER(vp)]
     L.dvo_b200_sharded_destroy.argtypes = [vp]
     L.dvo_b200_sharded_num_shards.argtypes = [vp]
@@ -258,6 +281,44 @@ class Pyramid:
             self.release()
         except Exception:
             pass
+
+
+class Selection:
+    """Owning handle of a dvo_b200_selection (dvo::core::PointSelection with its own predicate and mask).  Keeps the Python
+    Pyramid it was built from alive too, although the selection itself retains the device pyramid."""
+
+    def __init__(self, engine: "Engine", handle: int, pyramid: Pyramid):
+        self.engine, self.handle, self.pyramid = engine, handle, pyramid
+
+    def download(self, level: int):
+        """(S, mask[h, w] uint8): the number of selected points of the level and where they are."""
+        w, h, _ = self.pyramid.level_info(level)
+        mask = np.zeros((h, w), dtype=np.uint8)
+        cnt = C.c_int64()
+        ctx = self.engine.ctx if self.engine is not None else None
+        rc = load_library().dvo_b200_selection_download(ctx, self.handle, level, C.byref(cnt), mask.ctypes.data_as(C.POINTER(C.c_uint8)))
+        if rc != 0:
+            raise RuntimeError(f"dvo_b200_selection_download: status {rc}")
+        return cnt.value, mask
+
+    def release(self):
+        if self.handle:
+            load_library().dvo_b200_selection_release(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.release()
+        except Exception:
+            pass
+
+
+def _reference_handles(refs):
+    """(handles, selected): pyramids or selections as references of one batch, not mixed."""
+    sel = [isinstance(r, Selection) for r in refs]
+    if any(sel) and not all(sel):
+        raise ValueError("references of one batch are all Pyramids or all Selections")
+    return (C.c_void_p * len(refs))(*[r.handle for r in refs]), all(sel)
 
 
 class Engine:
@@ -362,14 +423,66 @@ class Engine:
         self.synchronize()
         return Pyramid(self, out.value)
 
+    # ---- point selections ----
+    def selection(self, pyramid: Pyramid, predicate: int = PREDICATE_GRADIENT_THRESHOLD, ti: float = 0.0, td: float = 0.0,
+                  masks=None) -> Selection:
+        """dvo_b200_selection_create: a selection of `pyramid` by `predicate` (PREDICATE_*; ti / td for the gradient
+        threshold), optionally restricted by host masks: one [h_l, w_l] array per level (nonzero = allowed) or None for a
+        level without mask.  level_masks() derives them from a level-0 mask."""
+        n = pyramid.num_levels
+        keep, arr = [], None
+        if masks is not None:
+            if len(masks) != n:
+                raise ValueError(f"masks: {n} levels expected, got {len(masks)}")
+            arr = (C.c_void_p * n)()
+            for l, m in enumerate(masks):
+                if m is None:
+                    continue
+                w, h, _ = pyramid.level_info(l)
+                a = np.ascontiguousarray(np.asarray(m) != 0, dtype=np.uint8)
+                if a.shape != (h, w):
+                    raise ValueError(f"mask of level {l}: shape {a.shape}, expected {(h, w)}")
+                keep.append(a)
+                arr[l] = a.ctypes.data
+        out = C.c_void_p()
+        self._check(self.lib.dvo_b200_selection_create(self.ctx, pyramid.handle, int(predicate), float(ti), float(td), arr, C.byref(out)))
+        return Selection(self, out.value, pyramid)
+
+    def selections_from_tensors(self, pyramids, masks=None, predicate: int = PREDICATE_GRADIENT_THRESHOLD, ti: float = 0.0,
+                                td: float = 0.0) -> list[Selection]:
+        """dvo_b200_selection_create_device_batch: one selection per pyramid in one build.  masks: None, or a CUDA
+        uint8 / bool tensor [n, h, w] of level-0 masks (nonzero = allowed) at any strides with unit stride along a row,
+        read in place; coarser levels subsample it like the depth.  Ordered after the current torch stream; the masks are
+        marked as used on the context's stream."""
+        import torch
+        n = len(pyramids)
+        ph = (C.c_void_p * n)(*[p.handle for p in pyramids])
+        ptr, row, img = None, 0, 0
+        ext = self._torch_stream()
+        if masks is not None:
+            self._check_on_device(masks, "masks")
+            if masks.dtype not in (torch.uint8, torch.bool) or masks.dim() != 3 or masks.shape[0] != n:
+                raise ValueError(f"masks: uint8 / bool [{n},h,w] expected, got {masks.dtype} {tuple(masks.shape)}")
+            if masks.stride(2) != 1:
+                raise ValueError("masks need unit stride along a row")
+            ptr, row = masks.data_ptr(), masks.stride(1)
+            img = masks.stride(0) if n > 1 else masks.shape[1] * row
+            ext.wait_stream(torch.cuda.current_stream(masks.device))
+        out = (C.c_void_p * n)()
+        self._check(self.lib.dvo_b200_selection_create_device_batch(self.ctx, n, ph, int(predicate), float(ti), float(td), ptr, row, img, out))
+        if masks is not None:
+            masks.record_stream(ext)
+        return [Selection(self, out[i], pyramids[i]) for i in range(n)]
+
     # ---- alignment ----
     def match(self, ref: Pyramid, cur: Pyramid, cfg: Config, T_init=None, with_iterations: bool = False) -> Result:
         return self.match_batch([ref], [cur], cfg, None if T_init is None else [T_init], with_iterations)[0]
 
     def match_batch(self, refs, curs, cfg: Config, T_init=None, with_iterations: bool = False, raw: bool = False):
+        """refs: Pyramids (their built-in selection with cfg's thresholds) or Selections (their own predicate and mask)."""
         n = len(refs)
         assert n == len(curs) and n > 0
-        rh = (C.c_void_p * n)(*[p.handle for p in refs])
+        rh, selected = _reference_handles(refs)
         ch = (C.c_void_p * n)(*[p.handle for p in curs])
         T = None
         if T_init is not None:
@@ -380,9 +493,9 @@ class Engine:
         if with_iterations:
             max_log = (cfg.first_level - cfg.last_level + 1) * (cfg.max_iterations_per_level + 1)
             log = (IterationStats * (n * max_log))()
-        self._check(self.lib.dvo_b200_match_batch(self.ctx, C.byref(cfg), n, rh, ch,
-                                                  T.ctypes.data_as(C.POINTER(C.c_double)) if T is not None else None,
-                                                  res, log, max_log))
+        fn = self.lib.dvo_b200_match_batch_selected if selected else self.lib.dvo_b200_match_batch
+        self._check(fn(self.ctx, C.byref(cfg), n, rh, ch, T.ctypes.data_as(C.POINTER(C.c_double)) if T is not None else None,
+                       res, log, max_log))
         if raw:
             return res
         out = []
@@ -445,7 +558,8 @@ class Engine:
     def match_batch_enqueue(self, refs, curs, cfg: Config, T_init=None):
         """dvo_b200_match_batch_enqueue: returns a uint8 CUDA tensor [n, sizeof(dvo_b200_result)] of result records,
         ordered onto the current torch stream; the host does not wait for the GPU.  T_init: CUDA float64 [n,4,4]
-        (Result.Transformation on entry, read iff cfg.use_initial_estimate).  result_transformations() views the poses."""
+        (Result.Transformation on entry, read iff cfg.use_initial_estimate).  result_transformations() views the poses.
+        refs: Pyramids or Selections, as for match_batch."""
         import torch
         n = len(refs)
         assert n == len(curs) and n > 0
@@ -458,12 +572,12 @@ class Engine:
                 raise ValueError(f"T_init: float64 [{n},4,4] expected, got {T_init.dtype} {tuple(T_init.shape)}")
             T = T_init.contiguous()
         records = torch.empty((n, C.sizeof(CResult)), dtype=torch.uint8, device=dev)
-        rh = (C.c_void_p * n)(*[p.handle for p in refs])
+        rh, selected = _reference_handles(refs)
         ch = (C.c_void_p * n)(*[p.handle for p in curs])
         ext = self._torch_stream()
         ext.wait_stream(cur)
-        self._check(self.lib.dvo_b200_match_batch_enqueue(self.ctx, C.byref(cfg), n, rh, ch, T.data_ptr() if T is not None else None,
-                                                          records.data_ptr()))
+        fn = self.lib.dvo_b200_match_batch_selected_enqueue if selected else self.lib.dvo_b200_match_batch_enqueue
+        self._check(fn(self.ctx, C.byref(cfg), n, rh, ch, T.data_ptr() if T is not None else None, records.data_ptr()))
         records.record_stream(ext)
         if T is not None:
             T.record_stream(ext)

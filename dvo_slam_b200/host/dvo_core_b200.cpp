@@ -254,11 +254,78 @@ bool DenseTracker::match(core::RgbdImagePyramid& reference, core::RgbdImagePyram
   return match(reference_selection_, current, result);
 }
 bool DenseTracker::match(core::PointSelection& reference, core::RgbdImagePyramid& current, Result& result) {
-  std::vector<core::RgbdImagePyramid*> refs(1, &reference.getRgbdImagePyramid()), curs(1, &current);
+  std::vector<core::PointSelection*> refs(1, &reference);
+  std::vector<core::RgbdImagePyramid*> curs(1, &current);
   std::vector<Result> results(1, result);
   bool ok = matchBatch(refs, curs, results);
   result = results[0];
   return ok;
+}
+
+// The tracker's own selection, or a gradient-threshold predicate with the configured thresholds: the pyramid's built-in
+// selection is exactly that (every call of dvo_slam).  Anything else gets a device selection of its own.
+bool DenseTracker::usesOwnSelection(const core::PointSelection& reference) const {
+  if (&reference == &reference_selection_) return true;
+  const core::ValidPointAndGradientThresholdPredicate* g =
+      dynamic_cast<const core::ValidPointAndGradientThresholdPredicate*>(&reference.predicate());
+  return g && g->intensity_threshold == cfg.IntensityDerivativeThreshold && g->depth_threshold == cfg.DepthDerivativeThreshold;
+}
+
+// PointSelection::select with the selection's own predicate (point_selection.cpp:89-152), as a device selection cached in
+// the PointSelection.  The two predicates of the reference map to their device forms; any other predicate is evaluated
+// here on every level -- isPointOk(x, y, z, idx, idy, zdx, zdy) with z the true depth of the level (the level-0 depth
+// subsampled) and the gradients of the device pyramid -- and handed over as MASK_ONLY masks.
+dvo_b200_selection* DenseTracker::deviceSelection(dvo_b200_ctx* ctx, core::PointSelection& reference) {
+  core::RgbdImagePyramid& pyr = reference.getRgbdImagePyramid();
+  dvo_b200_pyramid* p = pyr.device(ctx, cfg.getNumLevels());
+  if (dvo_b200_selection* s = reference.cachedDeviceSelection(p)) return s;
+  const core::PointSelectionPredicate& pred = reference.predicate();
+  const core::ValidPointAndGradientThresholdPredicate* g = dynamic_cast<const core::ValidPointAndGradientThresholdPredicate*>(&pred);
+  dvo_b200_selection* s = 0;
+  int rc;
+  if (g)
+    rc = dvo_b200_selection_create(ctx, p, DVO_B200_PREDICATE_GRADIENT_THRESHOLD, g->intensity_threshold, g->depth_threshold, 0, &s);
+  else if (dynamic_cast<const core::ValidPointPredicate*>(&pred))
+    rc = dvo_b200_selection_create(ctx, p, DVO_B200_PREDICATE_VALID_POINT, 0.f, 0.f, 0, &s);
+  else {
+    const int levels = dvo_b200_pyramid_num_levels(p);
+    const cv::Mat& depth0 = pyr.level(0).depth;
+    std::vector<std::vector<uint8_t> > masks(static_cast<size_t>(levels));
+    std::vector<const uint8_t*> ptrs(static_cast<size_t>(levels));
+    for (int l = 0; l < levels; ++l) {
+      int w = 0, h = 0;
+      float K[4];
+      dvo_b200_pyramid_level_info(p, l, &w, &h, K);
+      const size_t N = size_t(w) * h;
+      std::vector<float> planes(6 * N);
+      rc = dvo_b200_pyramid_download(ctx, p, l, planes.data());
+      if (rc != 0) throw std::runtime_error(std::string("dvo_b200_pyramid_download: ") + dvo_b200_last_error(ctx));
+      std::vector<uint8_t>& m = masks[size_t(l)];
+      m.resize(N);
+      for (int y = 0; y < h; ++y)
+        for (int x = 0; x < w; ++x) {
+          const size_t i = size_t(y) * w + x;
+          const float z = depth0.at<float>(y << l, x << l);
+          m[i] = pred.isPointOk(size_t(x), size_t(y), z, planes[2 * N + i], planes[3 * N + i], planes[4 * N + i], planes[5 * N + i]) ? 1 : 0;
+        }
+      ptrs[size_t(l)] = m.data();
+    }
+    rc = dvo_b200_selection_create(ctx, p, DVO_B200_PREDICATE_MASK_ONLY, 0.f, 0.f, ptrs.data(), &s);
+  }
+  if (rc != 0) throw std::runtime_error(std::string("dvo_b200_selection_create: ") + dvo_b200_last_error(ctx));
+  reference.cacheDeviceSelection(p, s);
+  return s;
+}
+
+bool DenseTracker::matchBatch(const std::vector<core::PointSelection*>& references, const std::vector<core::RgbdImagePyramid*>& currents,
+                              std::vector<Result>& results) {
+  std::vector<core::RgbdImagePyramid*> pyrs(references.size());
+  bool own = true;
+  for (size_t i = 0; i < references.size(); ++i) {
+    pyrs[i] = &references[i]->getRgbdImagePyramid();
+    own = own && usesOwnSelection(*references[i]);
+  }
+  return runBatch(pyrs, own ? 0 : &references, currents, results);
 }
 
 static void fill_result(const dvo_b200_result& r, const dvo_b200_iteration_stats* its, DenseTracker::Result& out) {
@@ -304,6 +371,13 @@ static void fill_result(const dvo_b200_result& r, const dvo_b200_iteration_stats
 
 bool DenseTracker::matchBatch(const std::vector<core::RgbdImagePyramid*>& references, const std::vector<core::RgbdImagePyramid*>& currents,
                               std::vector<Result>& results) {
+  return runBatch(references, 0, currents, results);
+}
+
+// selections == 0: every pair against its reference pyramid's built-in selection (cfg's thresholds); else pair i against
+// the device selection of (*selections)[i]
+bool DenseTracker::runBatch(const std::vector<core::RgbdImagePyramid*>& references, const std::vector<core::PointSelection*>* selections,
+                            const std::vector<core::RgbdImagePyramid*>& currents, std::vector<Result>& results) {
   const size_t n = references.size();
   if (n == 0 || currents.size() != n) return false;
   results.resize(n);
@@ -330,8 +404,16 @@ bool DenseTracker::matchBatch(const std::vector<core::RgbdImagePyramid*>& refere
   std::vector<dvo_b200_result> raw(n);
   const int max_log = collect_iterations_ ? (cfg.FirstLevel - cfg.LastLevel + 1) * (cfg.MaxIterationsPerLevel + 1) : 0;
   std::vector<dvo_b200_iteration_stats> log(size_t(max_log) * n);
-  int rc = dvo_b200_match_batch(ctx, &c, int(n), r.data(), q.data(), cfg.UseInitialEstimate ? T.data() : 0, raw.data(),
-                                max_log ? log.data() : 0, max_log);
+  int rc;
+  if (selections) {   // match(PointSelection&, ...): the selection's predicate decides, not cfg's thresholds
+    std::vector<dvo_b200_selection*> sel(n);
+    for (size_t i = 0; i < n; ++i) sel[i] = deviceSelection(ctx, *(*selections)[i]);
+    rc = dvo_b200_match_batch_selected(ctx, &c, int(n), sel.data(), q.data(), cfg.UseInitialEstimate ? T.data() : 0, raw.data(),
+                                       max_log ? log.data() : 0, max_log);
+  } else {
+    rc = dvo_b200_match_batch(ctx, &c, int(n), r.data(), q.data(), cfg.UseInitialEstimate ? T.data() : 0, raw.data(),
+                              max_log ? log.data() : 0, max_log);
+  }
   if (rc != 0) throw std::runtime_error(std::string("dvo_b200_match_batch: ") + dvo_b200_last_error(ctx));
   for (size_t i = 0; i < n; ++i) fill_result(raw[i], max_log ? &log[size_t(max_log) * i] : 0, results[i]);
   return true;   // the reference's match() always returns true (dense_tracking.cpp:135,375)

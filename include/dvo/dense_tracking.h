@@ -103,12 +103,19 @@ class DenseTracker {
   // and keyframe_graph.cpp:587-590).  results[i].Transformation is the initial guess on entry. ---
   bool matchBatch(const std::vector<core::RgbdImagePyramid*>& references, const std::vector<core::RgbdImagePyramid*>& currents,
                   std::vector<Result>& results);
+  // the same against PointSelections, each with its own predicate (match(PointSelection&, ...) for n pairs)
+  bool matchBatch(const std::vector<core::PointSelection*>& references, const std::vector<core::RgbdImagePyramid*>& currents,
+                  std::vector<Result>& results);
 
   // per-iteration statistics are copied back only when requested (they are optional in the C ABI)
   void collectIterationStatistics(bool on) { collect_iterations_ = on; }
 
  private:
   dvo_b200_ctx* context();
+  bool usesOwnSelection(const core::PointSelection& reference) const;
+  dvo_b200_selection* deviceSelection(dvo_b200_ctx* ctx, core::PointSelection& reference);
+  bool runBatch(const std::vector<core::RgbdImagePyramid*>& references, const std::vector<core::PointSelection*>* selections,
+                const std::vector<core::RgbdImagePyramid*>& currents, std::vector<Result>& results);
   Config cfg;
   dvo_b200_ctx* ctx_;
   bool collect_iterations_;

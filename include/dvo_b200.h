@@ -95,6 +95,7 @@ typedef struct dvo_b200_result {
 
 typedef struct dvo_b200_ctx dvo_b200_ctx;          /* one per host thread / CUDA stream */
 typedef struct dvo_b200_pyramid dvo_b200_pyramid;  /* device mirror of dvo::core::RgbdImagePyramid */
+typedef struct dvo_b200_selection dvo_b200_selection;  /* dvo::core::PointSelection of one pyramid (see below) */
 
 /* ---- context ------------------------------------------------------------------------------ */
 int dvo_b200_abi_version(void);
@@ -215,6 +216,53 @@ int dvo_b200_match_batch_device(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, i
 int dvo_b200_match_batch_enqueue(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int32_t n,
                                  dvo_b200_pyramid* const* references, dvo_b200_pyramid* const* currents,
                                  const double* d_T_init, void* d_results);
+
+/* ---- reference point selections (dvo::core::PointSelection with its own predicate, point_selection.h:39-124) -----------
+ * A selection is a device object of its own, separate from the pyramid's built-in selection (the one cfg's thresholds and
+ * dvo_b200_pyramid_select set): the reference points of every level of one pyramid, chosen by a predicate and optionally
+ * restricted by a per-pixel mask (exclude dynamic objects, the robot's body, saturated regions).  It retains its pyramid
+ * and may outlive the caller's pyramid handle and the context that built it.  Any number of selections of one pyramid can
+ * be aligned against at the same time, from any context.  Memory: its own copy of the reference tile records (about
+ * 7.4 MB at 640x480, 5 levels) from the context's slab pool. */
+typedef enum dvo_b200_predicate {
+  DVO_B200_PREDICATE_GRADIENT_THRESHOLD = 0,  /* ValidPointAndGradientThresholdPredicate(ti, td) (point_selection.h:52-67)  */
+  DVO_B200_PREDICATE_VALID_POINT = 1,         /* ValidPointPredicate: z, zdx, zdy not NaN (point_selection.h:39-47)        */
+  DVO_B200_PREDICATE_MASK_ONLY = 2            /* the mask alone decides; a pixel without valid depth still counts in S     */
+} dvo_b200_predicate;
+
+/* One selection of p.  level_masks: NULL (no mask), or p's number of levels entries, each NULL (every pixel allowed) or
+ * h_l*w_l HOST bytes of level l, nonzero = allowed.  The selected pixels are those where the predicate holds and the
+ * mask allows; the odd last one is dropped as computeResidualsSse does (dense_tracking_impl.cpp:169).  ti / td are read
+ * for GRADIENT_THRESHOLD only.  Asynchronous on the ctx stream; the masks are copied before the call returns. */
+int dvo_b200_selection_create(dvo_b200_ctx* ctx, dvo_b200_pyramid* p, int32_t predicate, float ti, float td,
+                              const uint8_t* const* level_masks, dvo_b200_selection** out);
+/* n selections of n pyramids of identical geometry in one build.  d_masks: NULL (no mask) or n level-0 masks of 8 bits per
+ * pixel in DEVICE memory, nonzero = allowed: pixel (x, y) of mask i at d_masks + i * image_bytes + y * row_bytes + x, row
+ * stride at least the width, image stride (read for n > 1) at least height x row stride.  Level l reads
+ * M_0(y << l, x << l), the subsample chain of the depth.  Host pointers, memory of another device and short strides are
+ * refused with DVO_B200_ERR_INVALID_ARGUMENT and build nothing.  Does not synchronise; the masks are read on the ctx
+ * stream (a caller that writes them on another stream makes the ctx stream wait first). */
+int dvo_b200_selection_create_device_batch(dvo_b200_ctx* ctx, int32_t n, dvo_b200_pyramid* const* pyramids, int32_t predicate,
+                                           float ti, float td, const void* d_masks, int64_t row_bytes, int64_t image_bytes,
+                                           dvo_b200_selection** out /* n handles */);
+int dvo_b200_selection_retain(dvo_b200_selection* s);
+int dvo_b200_selection_release(dvo_b200_selection* s);
+dvo_b200_pyramid* dvo_b200_selection_pyramid(dvo_b200_selection* s);   /* borrowed: the selection holds the reference */
+/* Number of selected points S of a level (PointSelection::select's point count) and, optionally, the h*w byte mask of the
+ * selected points (the odd last one included, as dvo_b200_pyramid_select reports it).  Synchronises; ctx may be NULL: the
+ * read then waits for the selection's build only. */
+int dvo_b200_selection_download(dvo_b200_ctx* ctx, const dvo_b200_selection* s, int32_t level, int64_t* count, uint8_t* mask);
+/* dvo_b200_match_batch / dvo_b200_match_batch_enqueue with pair i aligned against selection references[i] of its pyramid:
+ * DenseTracker::match(PointSelection& reference, current, result) (dense_tracking.cpp:131-376).  cfg's derivative
+ * thresholds are not read: the selection's predicate decides.  A selection equal to the pyramid's own selection gives
+ * the same result records byte for byte. */
+int dvo_b200_match_batch_selected(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int32_t n,
+                                  dvo_b200_selection* const* references, dvo_b200_pyramid* const* currents,
+                                  const double* T_init, dvo_b200_result* results,
+                                  dvo_b200_iteration_stats* iteration_stats, int32_t max_iteration_stats);
+int dvo_b200_match_batch_selected_enqueue(dvo_b200_ctx* ctx, const dvo_b200_config* cfg, int32_t n,
+                                          dvo_b200_selection* const* references, dvo_b200_pyramid* const* currents,
+                                          const double* d_T_init, void* d_results);
 
 /* ---- one process, several GPUs (SURVEY.md 8e) ----------------------------------------------------
  * The reference's batch producers are single-process C++ loops over independent match() calls

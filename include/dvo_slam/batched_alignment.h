@@ -37,6 +37,24 @@ inline bool matchKeyframeAndOdometry(dvo::DenseTracker& tracker, dvo::core::Rgbd
   return ok;
 }
 
+// The same with the reference points of LocalTracker's own PointSelections (local_tracker.cpp:59-61,180-184: the keyframe's
+// and the previous frame's selection, each with the tracker's predicate), so that their predicate reaches the device.
+inline bool matchKeyframeAndOdometry(dvo::DenseTracker& tracker, dvo::core::PointSelection& keyframe,
+                                     dvo::core::PointSelection& previous_frame, dvo::core::RgbdImagePyramid& current,
+                                     dvo::DenseTracker::Result& r_keyframe, dvo::DenseTracker::Result& r_odometry) {
+  std::vector<dvo::core::PointSelection*> references;
+  std::vector<dvo::core::RgbdImagePyramid*> currents;
+  references.push_back(&keyframe); references.push_back(&previous_frame);
+  currents.push_back(&current); currents.push_back(&current);
+  std::vector<dvo::DenseTracker::Result> results(2);
+  results[0].Transformation = r_keyframe.Transformation;
+  results[1].Transformation = r_odometry.Transformation;
+  const bool ok = tracker.matchBatch(references, currents, results);
+  r_keyframe = results[0];
+  r_odometry = results[1];
+  return ok;
+}
+
 // The tracking loop of ConstraintProposalValidator::validate.  ProposalPtrVector is any sequence of pointer-likes
 // to objects with the members the reference's ConstraintProposal has: Reference->image(), Current->image()
 // (RgbdImagePyramid::Ptr), InitialTransformation and TrackingResult (constraint_proposal.h).
